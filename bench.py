@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: leg-frames/s of the 4-stage sequential leg IK (+FK) on synthetic pose data.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--trials T] [--frames F] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--trials T] [--frames F] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (stages 1-4 + 9-row FK) over T trials x 6 legs x F frames per GPU
 (default T = 1000, F = 1000: BASELINE.json config "synthetic 1k trials x 1000 frames x 6 legs on 1 B200").
@@ -22,6 +22,11 @@ The same line carries
 --impl reference times that CPU implementation alone, with every host core, on bounded samples of the same
 workload (see DESIGN.md: the reference's own per-frame chain rebuild needs ikpy/sympy, which is not
 installable offline; the oracle is its arithmetic without that overhead, i.e. a faster stand-in).
+
+--dump-outputs DIR writes what the last timed step returned (rank 0: the angles and FK of `value`'s solve_device call)
+as DIR/angles.npy (chains, frames, 7) and DIR/fk.npy (chains, frames, 9, 3), float32.  The synthetic pose is seeded, so
+the same arguments give the same inputs and two builds can be compared output for output.  Outputs above DUMP_BYTES are
+sampled with a fixed seed: whole chains while one fits, else a subset of frames as well (sorted indices).
 """
 import argparse
 import json
@@ -42,6 +47,7 @@ METRIC = "leg-frames/sec, 4-stage seq IK"
 UNIT = "leg-frames/s"
 ALG_BYTES_PER_LEG_FRAME = 60 + 28 + 108          # pose in + angles out + FK out, fp32 (SURVEY.md 8d / DESIGN.md)
 ALG_FLOP_PER_LEG_FRAME = 14.5e3                   # nominal full-chain model of SURVEY.md 8d (DESIGN.md)
+DUMP_BYTES = 60_000_000                           # --dump-outputs: array bytes in all (64 MB less room for the .npy headers)
 
 
 # --------------------------------------------------------------------------------------------- CPU oracle legs
@@ -134,6 +140,28 @@ def workload_config(args, note=None):
     if note:
         cfg["note"] = note
     return cfg
+
+
+def sample_outputs(angles, fk):
+    """Device copies of a fixed, seeded sample of (angles, fk) of at most DUMP_BYTES, enqueued behind the step that wrote
+    them, so that later calls into the same session buffers do not change what is dumped."""
+    import torch
+    n_chain, n_frame = angles.shape[:2]
+    lf_budget = DUMP_BYTES // (angles[0, 0].nbytes + fk[0, 0].nbytes)
+    n_c = max(1, min(n_chain, lf_budget // n_frame))
+    n_f = min(n_frame, lf_budget // n_c)
+    rng = np.random.default_rng(0)
+    chains = torch.from_numpy(np.sort(rng.choice(n_chain, n_c, replace=False))).to(angles.device)
+    frames = torch.from_numpy(np.sort(rng.choice(n_frame, n_f, replace=False))).to(angles.device)
+    return {name: t.index_select(0, chains).index_select(1, frames) for name, t in (("angles", angles), ("fk", fk))}
+
+
+def write_outputs(out_dir, outputs):
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for name, t in outputs.items():
+        np.save(out / f"{name}.npy", t.cpu().numpy())
+    print(f"bench.py: wrote {', '.join(f'{n}.npy {tuple(t.shape)}' for n, t in outputs.items())} to {out}", file=sys.stderr)
 
 
 class ClockSampler(threading.Thread):
@@ -284,6 +312,7 @@ def run_ours(args):
         sampler.start()
     ms_total = timed(lambda: sess.solve_device(want_stats=False), args.steps)
     ms_step = ms_total / args.steps
+    dumped = sample_outputs(sess.d_angles, sess.d_fk) if args.dump_outputs and rank == 0 else None
     # ---- end to end through the public batched call with host buffers
     for _ in range(2):
         sess.solve_host(host_pose, n_chunks=args.chunks)
@@ -405,6 +434,8 @@ def run_ours(args):
                 secondary[name] = {"error": repr(exc)[:300]}
             torch.cuda.empty_cache()
 
+    if dumped is not None:
+        write_outputs(args.dump_outputs, dumped)
     if rank == 0:
         peaks = {}
         try:
@@ -514,9 +545,15 @@ def main():
     ap.add_argument("--no-secondary", action="store_true", help="skip the secondary records (config 2 dict API, stream kernels, config 5)")
     ap.add_argument("--config5-trials", type=int, default=100)
     ap.add_argument("--config5-frames", type=int, default=100000)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the angles and FK of the last timed step as DIR/*.npy (seeded sample above 64 MB)")
     ap.add_argument("--cpu-baseline-only", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--cpu-procs", type=int, default=6, help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours (the reference arm returns no arrays)")
     if args.cpu_baseline_only:
         done, times = oracle_throughput(1, args.cpu_frames, args.cpu_procs)
         t0 = time.perf_counter()

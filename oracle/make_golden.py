@@ -32,6 +32,9 @@ Fixtures
                      inputs and converter outputs, for the batched loader's key-order semantics
   synthetic_long.npz trial 5, legs RM and LH, 2000 frames: oracle angles (float32) -- a long warm-start chain that spans
                      many of the kernel's 64-frame resync periods
+  reference_constants.json
+                     INITIAL_ANGLES, BOUNDS, NMF_SIZE, PTS2ALIGN and NMF_TEMPLATE of the reference's seqikpy/data.py
+                     (`--constants-only`): key order kept, floats written exactly
 """
 import argparse
 import os
@@ -308,8 +311,27 @@ def make_loader_fixture():
     print("loader.npz", {k: v.shape for k, v in out.items() if k.endswith(("_table", "_array")) or "_ref_RF" in k})
 
 
+REFERENCE_CONSTANTS = ("INITIAL_ANGLES", "BOUNDS", "NMF_SIZE", "PTS2ALIGN", "NMF_TEMPLATE")
+
+
+def make_constants_fixture(data_module):
+    """The public constants of `data_module` (the reference's seqikpy.data) as JSON; json writes floats by repr, so the
+    values read back bit for bit."""
+    import json
+
+    def plain(v):
+        if isinstance(v, dict):
+            return {str(k): plain(x) for k, x in v.items()}
+        return np.asarray(v).tolist()
+    out = {name: plain(getattr(data_module, name)) for name in REFERENCE_CONSTANTS}
+    (GOLD / "reference_constants.json").write_text(json.dumps(out, indent=1) + "\n")
+
+
 if __name__ == "__main__":
-    if "--loader-only" in sys.argv:
+    if "--constants-only" in sys.argv:
+        import seqikpy.data as RD
+        make_constants_fixture(RD)
+    elif "--loader-only" in sys.argv:
         make_loader_fixture()
     else:
         main()

@@ -122,19 +122,17 @@ def test_synthetic_workload_is_reproducible_and_feasible(synthetic_gold):
     assert chains.shape == (12, 20, 5, 3) and np.array_equal(chains[7, 3], S.make_trial(1, 20)[3, 1].astype(np.float32))
 
 
-def test_constants_equal_reference_when_available():
-    """Cross-check against the reference checkout where it exists (the build container); skipped on the GPU box."""
-    import os
-    import sys
-    if not os.path.isdir("/root/reference/seqikpy"):
-        pytest.skip("no reference checkout here")
-    sys.path.insert(0, "/root/reference")
-    try:
-        from seqikpy import data as RD
-    finally:
-        sys.path.remove("/root/reference")
+def test_constants_equal_reference():
+    """The public constants equal the reference's seqikpy/data.py, stored in tests/golden/reference_constants.json
+    (oracle/make_golden.py --constants-only); its key-point names also travel in loader.npz."""
+    import json
+    import conftest
+    ref_all = json.loads((conftest.GOLDEN / "reference_constants.json").read_text())
+    loader = np.load(conftest.GOLDEN / "loader.npz")
+    for seg in loader["anipose_segments"]:
+        assert D.PTS2ALIGN[str(seg)] == [str(k) for k in loader[f"anipose_kps_{seg}"]], seg
     for name in ("INITIAL_ANGLES", "BOUNDS", "NMF_SIZE", "PTS2ALIGN", "NMF_TEMPLATE"):
-        ours, ref = getattr(D, name), getattr(RD, name)
+        ours, ref = getattr(D, name), ref_all[name]
         assert list(ours.keys()) == list(ref.keys()), name
         for k in ours:
             if isinstance(ours[k], dict):
@@ -145,10 +143,9 @@ def test_constants_equal_reference_when_available():
 
 def test_raw_format_converters(locomotion, tmp_path):
     """Converters feeding AlignPose (reference alignment.py:103-226): shapes, values, and agreement with the reference's
-    own functions where its checkout is present."""
-    import os
+    own functions on the inputs and outputs of them stored in tests/golden/loader.npz."""
     import pickle
-    import sys
+    import conftest
     from seqikpy_b200.alignment import (AlignPose, convert_from_anipose_to_dict, convert_from_df3d_to_dict,
                                         convert_from_df3dpp_to_dict)
     rng = np.random.default_rng(0)
@@ -174,16 +171,18 @@ def test_raw_format_converters(locomotion, tmp_path):
     assert al.pose_data_dict["RF_leg"].shape == (n, 5, 3) and al.include_claw is False
     with pytest.raises(FileNotFoundError):
         AlignPose.from_file_path(main_dir=tmp_path, file_name="nothing.*", legs_list=["RF"])
-    if os.path.isdir("/root/reference/seqikpy"):
-        sys.path.insert(0, "/root/reference")
-        try:
-            from seqikpy import alignment as RA
-        finally:
-            sys.path.remove("/root/reference")
-        ref = RA.convert_from_anipose_to_dict(table, D.PTS2ALIGN)
-        assert all(np.array_equal(ref[k], conv[k]) for k in ref)
-        assert all(np.array_equal(v, dpp[k]) for k, v in RA.convert_from_df3dpp_to_dict(pp, ["RF_leg", "LM_leg"]).items())
-        assert all(np.array_equal(v, d3[k]) for k, v in RA.convert_from_df3d_to_dict(arr, idx).items())
+    gold = np.load(conftest.GOLDEN / "loader.npz")
+    table_r = {str(k): gold["anipose_table"][i] for i, k in enumerate(gold["anipose_columns"])}
+    pts_r = {str(s): [str(k) for k in gold[f"anipose_kps_{s}"]] for s in gold["anipose_segments"]}
+    conv_r = convert_from_anipose_to_dict(table_r, pts_r)
+    assert list(conv_r.keys()) == list(pts_r.keys()) and all(np.array_equal(v, gold[f"anipose_ref_{k}"]) for k, v in conv_r.items())
+    segs = [f"{leg}_leg" for leg in ("RF", "RM", "RH", "LF", "LM", "LH")]
+    d3_r = convert_from_df3d_to_dict(gold["df3d_array"], {s: gold[f"df3d_idx_{s}"] for s in segs})
+    assert all(np.array_equal(d3_r[s], gold[f"df3d_ref_{s}"]) for s in segs)
+    pp_r = {s: {kp: {"raw_pos_aligned": gold[f"df3dpp_raw_{s}"][j]} for j, kp in enumerate(("Coxa", "Femur", "Tibia", "Tarsus", "Claw"))}
+            for s in segs}
+    dpp_r = convert_from_df3dpp_to_dict(pp_r, segs)
+    assert list(dpp_r.keys()) == segs and all(np.array_equal(dpp_r[s], gold[f"df3dpp_ref_{s}"]) for s in segs)
 
 
 def test_interpolate_joint_angles_needs_the_device():
@@ -222,56 +221,3 @@ def test_leg_ik_class_exposes_the_solver_mode():
     assert LegInvKinSeq(pose, ch, D.INITIAL_ANGLES, log_level="ERROR", reference_iterates=True).flags == N.FLAG_REFERENCE_ITERATES
     assert LegInvKinSeq(pose, ch, D.INITIAL_ANGLES, log_level="ERROR", flags=0x7F).flags == 0x7F
 
-
-def test_reference_visualization_loader_reads_our_pickles(tmp_path, grooming_leg, grooming_head):
-    """SURVEY 8(f4): the reference's plotting code consumes the pickles through visualization.load_grid_plot_data
-    (visualization.py:191-213).  The REFERENCE's own function (imported from /root/reference with matplotlib stubbed out --
-    it is not installed here and the loader does not use it) reads the files our writers produce, under the reference's file
-    names, and finds the keys and shapes its consumers index.  Skipped where the reference checkout is absent (GPU box)."""
-    import sys
-    import types
-    from pathlib import Path
-    ref_root = Path("/root/reference")
-    if not (ref_root / "seqikpy" / "visualization.py").exists():
-        pytest.skip("reference checkout not available")
-    class _Stub(types.ModuleType):                                  # any attribute (plt.Axes in annotations, GridSpec, ...) is a dummy class
-        def __getattr__(self, name):
-            if name.startswith("__"):
-                raise AttributeError(name)
-            return type(name, (), {})
-    stubs = {}
-    for name in ("matplotlib", "matplotlib.animation", "matplotlib.gridspec", "matplotlib.pyplot", "matplotlib.backends",
-                 "matplotlib.backends.backend_agg"):
-        if name not in sys.modules:
-            stubs[name] = _Stub(name)
-    for name, mod in stubs.items():                                 # `import a.b as c` resolves b as an attribute of a
-        if "." in name and name.rsplit(".", 1)[0] in stubs:
-            setattr(stubs[name.rsplit(".", 1)[0]], name.rsplit(".", 1)[1], mod)
-    sys.modules.update(stubs)
-    sys.path.insert(0, str(ref_root))
-    try:
-        try:
-            from seqikpy import visualization as RV
-        except Exception as exc:                                   # e.g. cv2 missing
-            pytest.skip(f"reference visualization module not importable: {exc!r}")
-        # files exactly as our classes write them (export_path=): plain dicts of float64 arrays under the reference's names
-        leg = {str(k): grooming_leg["ref_angles"][i // 7][:, i % 7].astype(np.float64) for i, k in enumerate(grooming_leg["angle_keys"])}
-        head = {str(k): grooming_head["ref_angles"][i].astype(np.float64) for i, k in enumerate(grooming_head["keys"])}
-        aligned = {"RF_leg": grooming_leg["pose"][0], "LF_leg": grooming_leg["pose"][1], "R_head": grooming_head["r_head"],
-                   "L_head": grooming_head["l_head"], "Neck": grooming_head["neck"]}
-        save_file(tmp_path / "leg_joint_angles.pkl", leg)
-        save_file(tmp_path / "head_joint_angles.pkl", head)
-        save_file(tmp_path / "pose3d_aligned.pkl", aligned)
-        ja, pose = RV.load_grid_plot_data(tmp_path)                # head + leg files merged
-        assert list(ja.keys()) == list(head.keys()) + list(leg.keys()) and len(ja) == 21
-        assert pose["RF_leg"].shape == (6000, 5, 3) and pose["Neck"].shape == (1, 1, 3)
-        save_file(tmp_path / "body_joint_angles.pkl", {**head, **leg})
-        ja2, _ = RV.load_grid_plot_data(tmp_path)                  # the merged file takes precedence
-        assert list(ja2.keys()) == list(ja.keys()) and all(np.array_equal(ja2[k], ja[k]) for k in ja)
-        assert all(k.startswith("Angle_") and v.shape == (6000,) and v.dtype == np.float64 for k, v in ja2.items())
-    finally:
-        sys.path.remove(str(ref_root))
-        for name in stubs:
-            sys.modules.pop(name, None)
-        for name in [m for m in sys.modules if m == "seqikpy" or m.startswith("seqikpy.")]:
-            sys.modules.pop(name, None)
