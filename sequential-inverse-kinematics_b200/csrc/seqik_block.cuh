@@ -22,6 +22,9 @@
 // carried solve (tests/hostsim run_carried, leg_solve_pipe_kernel), so results are BIT-IDENTICAL to schedule 2; the
 // functions below restate warm_step() piecewise and are pinned to it by tests/test_host_core.py (host emulation of this
 // schedule against the serial one) and tests/test_gpu_parity.py (kernel against kernel).
+// The per-stage constants (stage_const), the serial stage step of the replay and of the first frame (serial_stage), the
+// frame rotation (rotate_stage) and the forward-kinematics rows (put_fk_joint) below are the kernels' code and the host
+// emulation's (tests/hostsim run_block) alike, so the CPU suite compiles and runs the same arithmetic as the GPU.
 #pragma once
 #include "seqik_core.cuh"
 
@@ -130,6 +133,94 @@ SK_HD int warm_case(bool enable, bool have_bt, bool one_var, R xp0, R xp1, const
     const bool ok_b = (N::abs_(b_x0 - xp0) < StageSolve<R>::ws_move_max()) & small_b2 & lim_ok_q & (cx1 - lb1s > m) & (ub1s - cx1 > m);
     x0 = b_x0; x1 = cx1;
     return ok_b ? (lo ? WC_LO : WC_HI) : WC_NONE;
+}
+
+// ---- the constants of one (chain, stage), derived from the chain's 32-float parameter row (include/seqik.h: segment
+// lengths 0..3, lower / upper limits 4..10 / 11..17, seed 18..24, null_sq 25..28).  SerialConst: what serial_stage() reads.
+// It stays these ten floats: the robust block kernel hands them to its out-of-line serial_stage_call through memory.
+template <typename R> struct SerialConst {
+    R L, lb0, ub0, lb1, ub1;            // segment length, limits of the first / second angle in the caller's terms
+    R sl0, cl0, su0, cu0;               // sin/cos of the first angle's limits (all zero without both: warm_guess says interior)
+    R nsq;                              // squared norm of the inert slots (StageSolve::null_sq)
+    SK_HD bool have_bt() const { return lb0 > -Num<R>::inf() && ub0 < Num<R>::inf(); }
+};
+template <typename R> struct StageConst : SerialConst<R> {
+    int ia, ib;                         // row indices of the first / second angle (stage 4 has one: ia = ib = 6)
+    R shift;                            // stage 1 is solved in the Rz Ry form: second angle x1 = b - pi/2
+    R lb1s, ub1s;                       // second angle's limits in that form
+    R lb0p, ub0p;                       // the first angle's limits as place1 leaves them (the value of a frame on a limit)
+};
+template <typename R> SK_HD R ld_param(const R* p) {
+#if defined(__CUDA_ARCH__)
+    return __ldg(p);
+#else
+    return *p;
+#endif
+}
+template <typename R> SK_HD StageConst<R> stage_const(const R* prm, int s) {
+    typedef Num<R> N;
+    const R inf = N::inf();
+    StageConst<R> k;
+    k.ia = 2 * s; k.ib = (s == 3) ? 6 : 2 * s + 1;
+    k.shift = (s == 0) ? R(1.57079632679489661923) : R(0);
+    k.lb0 = (s == 3) ? -inf : ld_param(prm + 4 + k.ia); k.ub0 = (s == 3) ? inf : ld_param(prm + 11 + k.ia);
+    k.lb1 = ld_param(prm + 4 + k.ib); k.ub1 = ld_param(prm + 11 + k.ib);
+    k.L = ld_param(prm + s); k.nsq = ld_param(prm + 25 + s);
+    k.lb1s = k.lb1 - k.shift; k.ub1s = k.ub1 - k.shift;
+    k.sl0 = k.cl0 = k.su0 = k.cu0 = R(0);
+    R v_;
+    if (k.have_bt()) { N::sincosv_(k.lb0, &k.sl0, &k.cl0, &v_); N::sincosv_(k.ub0, &k.su0, &k.cu0, &v_); }
+    k.lb0p = place1(k.lb0, k.lb0, k.ub0); k.ub0p = place1(k.ub0, k.lb0, k.ub0);
+    return k;
+}
+
+// ---- A <- A Rot_a(a) Ry(b) of stage s, from the sin/cos of its iterate in the Rz Ry form (stage 1: b = x1 + pi/2, so
+// sin b = cos x1 and cos b = -sin x1, as StageSolve::sin_b / cos_b)
+template <typename R> SK_HD Mat3<R> rotate_stage(const Mat3<R>& A, int s, R sa, R ca, R sb, R cb) {
+    const bool xy = s == 0;
+    return rotate_frame_sel(A, xy ? KIND_XY : KIND_ZY, sa, ca, xy ? cb : sb, xy ? -sb : cb);
+}
+
+// ---- the forward-kinematics rows of stage s's joint w in one leg-frame.  kFk 1, nine rows: 0-3 the origin o, 4 repeats 5,
+// 5 + s the joint of stage s (stage s writes rows s and 5 + s, stage 1 also row 4).  kFk 2, the joints only: row s.
+template <int kFk, typename R> SK_HD void put_fk_joint(R* fk, int s, const Vec3<R>& o, const Vec3<R>& w) {
+    if (kFk == 1) {
+        fk[3 * s] = o.x; fk[3 * s + 1] = o.y; fk[3 * s + 2] = o.z;
+        fk[15 + 3 * s] = w.x; fk[16 + 3 * s] = w.y; fk[17 + 3 * s] = w.z;
+        if (s == 0) { fk[12] = w.x; fk[13] = w.y; fk[14] = w.z; }
+    } else if (kFk == 2) { fk[3 * s] = w.x; fk[3 * s + 1] = w.y; fk[3 * s + 2] = w.z; }
+}
+
+// ---- one stage of one frame through the serial solver, exactly as run_carried / leg_solve_pipe_kernel run it for a carried
+// solve: the iterate (x0, x1: placed angles; sa..cb: their sin/cos) meets the target kt in the frame (A, piv) the earlier
+// stages of this frame built.  On return the iterate is the solve's final one, (A, piv) are those of the next stage, w is the
+// joint position, xb_out the second angle in the caller's terms.  The replay of the block kernel, the first-frame kernel and
+// the host emulation of the schedule run this code.
+template <typename R>
+SK_HD void serial_stage(int s, const SerialConst<R>& k, int gn_mask, bool esc, bool warm_ok, const Vec3<R>& kt, const Vec3<R>& o,
+                        Mat3<R>& A, Vec3<R>& piv, R& x0, R& x1, R& sa, R& ca, R& sb, R& cb, R& xb_out, Vec3<R>& w,
+                        uint32_t& nfev, int& worst) {
+    StageSolve<R> S;
+    S.set_problem(s == 0 ? KIND_XY : KIND_ZY, k.L, s == 3 ? R(0) : R(1), k.nsq, (s == 0) ? 4 : (s == 1) ? 6 : (s == 2) ? 8 : 9, stage_mode(gn_mask, s));
+    S.sl0 = k.sl0; S.cl0 = k.cl0; S.su0 = k.su0; S.cu0 = k.cu0;
+    S.have_bt = k.have_bt();
+    S.x0 = x0; S.x1 = x1; S.sa = sa; S.ca = ca; S.sb = sb; S.cb = cb;
+    const Vec3<R> rel = {(kt.x - o.x) - piv.x, (kt.y - o.y) - piv.y, (kt.z - o.z) - piv.z};
+    const Vec3<R> q3 = mulT(A, rel);
+    S.restart(q3, k.lb0, k.ub0, k.lb1, k.ub1, false, warm_ok);
+    for (;;) {
+        while (!S.done()) S.trip();
+        if (!(esc && S.escape())) break;
+    }
+    nfev += (uint32_t)S.nfev;
+    worst = (S.status == ST_MAXFEV && worst > ST_MAXFEV) ? ST_MAXFEV : worst;
+    worst = (S.status == ST_NONFINITE) ? ST_NONFINITE : worst;
+    const Vec3<R> Af = mul(A, S.res());
+    const Vec3<R> np_ = {(piv.x + rel.x) + Af.x, (piv.y + rel.y) + Af.y, (piv.z + rel.z) + Af.z};
+    w = {np_.x + o.x, np_.y + o.y, np_.z + o.z};
+    A = rotate_stage(A, s, S.sa, S.ca, S.sb, S.cb);
+    piv = np_;
+    x0 = S.x0; x1 = S.x1; sa = S.sa; ca = S.ca; sb = S.sb; cb = S.cb; xb_out = S.angle_b();
 }
 
 }  // namespace seqik

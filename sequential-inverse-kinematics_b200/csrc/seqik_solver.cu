@@ -299,7 +299,9 @@ __global__ void __launch_bounds__(32) leg_solve_pipe_kernel(LegArgs a, int cpw, 
 // ---------------------------------------------------------------------------------------------
 // schedule 3: frame-parallel blocks -- one warp per chain, 32 consecutive frames per pass (lane = frame)
 // ---------------------------------------------------------------------------------------------
-// The algorithm and why its results are bit-identical to schedule 2 are described in seqik_block.cuh.  Per warp:
+// The algorithm and why its results are bit-identical to schedule 2 are described in seqik_block.cuh, which also holds the
+// per-stage constants and the serial stage step of the replay and of the first frame: the host emulation of the schedule
+// (tests/hostsim run_block) compiles the same code.  Per warp:
 //   * the 32 x 60 B of key points of the NEXT block arrive by one bulk copy (cp.async.bulk -> mbarrier) while the current
 //     block is solved; angles (32 x 28 B) and forward kinematics (32 x 108 B) are staged in shared memory and leave by two
 //     bulk stores: every byte of the chain crosses the memory system once, in 128-byte lines (BASELINE.json north_star 2);
@@ -308,41 +310,10 @@ __global__ void __launch_bounds__(32) leg_solve_pipe_kernel(LegArgs a, int cpw, 
 // A CTA is one warp (no block-level barrier); the launch shapes the number of resident warps per SM with dynamic shared
 // memory so that the chains of a batch run in whole waves (seqik_leg_solve_f32).
 constexpr int BLK = 32;
-// One stage of one frame through the serial solver, exactly as hostsim run_carried / leg_solve_pipe_kernel run it for a carried
-// solve: the iterate (x0, x1: placed angles; sa..cb: their sin/cos) meets the target kt in the frame (A, piv) the earlier
-// stages of this frame built.  On return the iterate is the solve's final one, (A, piv) are those of the next stage, w is the
-// joint position.  Shared by the replay path of the block kernel and by the first-frame kernel.
-struct StageK { float L, lb0, ub0, lb1, ub1, sl0, cl0, su0, cu0, nsq; };
-__device__ __forceinline__ void serial_stage(int s, const StageK& k, int gn_mask, bool esc, bool warm_ok, const Vec3<float>& kt,
-                                             const Vec3<float>& o, Mat3<float>& A, Vec3<float>& piv, float& x0, float& x1,
-                                             float& sa, float& ca, float& sb, float& cb, float& xb_out, Vec3<float>& w,
-                                             uint32_t& nfev, int& worst) {
-    const float inf = Num<float>::inf();
-    StageSolve<float> S;
-    S.set_problem(s == 0 ? KIND_XY : KIND_ZY, k.L, s == 3 ? 0.f : 1.f, k.nsq, (s == 0) ? 4 : (s == 1) ? 6 : (s == 2) ? 8 : 9, stage_mode(gn_mask, s));
-    S.sl0 = k.sl0; S.cl0 = k.cl0; S.su0 = k.su0; S.cu0 = k.cu0;
-    S.have_bt = k.lb0 > -inf && k.ub0 < inf;
-    S.x0 = x0; S.x1 = x1; S.sa = sa; S.ca = ca; S.sb = sb; S.cb = cb;
-    const Vec3<float> rel = {(kt.x - o.x) - piv.x, (kt.y - o.y) - piv.y, (kt.z - o.z) - piv.z};
-    const Vec3<float> q3 = mulT(A, rel);
-    S.restart(q3, k.lb0, k.ub0, k.lb1, k.ub1, false, warm_ok);
-    for (;;) {
-        while (!S.done()) S.trip();
-        if (!(esc && S.escape())) break;
-    }
-    nfev += (uint32_t)S.nfev;
-    worst = (S.status == ST_MAXFEV && worst > ST_MAXFEV) ? ST_MAXFEV : worst;
-    worst = (S.status == ST_NONFINITE) ? ST_NONFINITE : worst;
-    const Vec3<float> Af = mul(A, S.res());
-    const Vec3<float> np_ = {(piv.x + rel.x) + Af.x, (piv.y + rel.y) + Af.y, (piv.z + rel.z) + Af.z};
-    w = {np_.x + o.x, np_.y + o.y, np_.z + o.z};
-    A = rotate_frame_sel(A, s == 0 ? KIND_XY : KIND_ZY, S.sa, S.ca, S.sin_b(), S.cos_b());
-    piv = np_;
-    x0 = S.x0; x1 = S.x1; sa = S.sa; ca = S.ca; sb = S.sb; cb = S.cb; xb_out = S.angle_b();
-}
-// The same as a real call (robust block kernel): the ~75 registers of the serial solver are then the callee's business and what
-// the kernel keeps across it is saved at the -- cold -- call site instead of being spilled where it is defined, in the hot pass.
-__device__ __noinline__ void serial_stage_call(int s, const StageK& k, int gn_mask, bool esc, bool warm_ok, const Vec3<float>& kt,
+// serial_stage (seqik_block.cuh) as a real call (robust block kernel): the ~75 registers of the serial solver are then the
+// callee's business and what the kernel keeps across it is saved at the -- cold -- call site instead of being spilled where it
+// is defined, in the hot pass.
+__device__ __noinline__ void serial_stage_call(int s, const SerialConst<float>& k, int gn_mask, bool esc, bool warm_ok, const Vec3<float>& kt,
                                                const Vec3<float>& o, Mat3<float>& A, Vec3<float>& piv, float& x0, float& x1,
                                                float& sa, float& ca, float& sb, float& cb, float& xb_out, Vec3<float>& w,
                                                uint32_t& nfev, int& worst) {
@@ -376,8 +347,6 @@ __global__ void __launch_bounds__(BLK) leg_first_frame_kernel(LegArgs a) {
     const float* kp = a.pose + c * a.pose_cs;
     float* ang = a.angles + c * a.ang_cs;
     float* fk = kFk ? a.fk + c * a.fk_cs : nullptr;
-    const float inf = Num<float>::inf();
-    const float half_pi = 1.57079632679489661923f;
     LoadMap map; map.init(a.affine, c);
     const bool esc = (a.gn_mask >> 4) & 1;
     const Vec3<float> o = map.apply({__ldg(kp), __ldg(kp + 1), __ldg(kp + 2)}, 0);
@@ -386,35 +355,23 @@ __global__ void __launch_bounds__(BLK) leg_first_frame_kernel(LegArgs a) {
     int worst = ST_GTOL;
 #pragma unroll 1
     for (int s = 0; s < 4; ++s) {
-        const int ia = 2 * s, ib = (s == 3) ? 6 : 2 * s + 1;
-        const float shift = (s == 0) ? half_pi : 0.f;
-        StageK k;
-        k.L = __ldg(prm + s); k.nsq = __ldg(prm + 25 + s);
-        k.lb0 = (s == 3) ? -inf : __ldg(prm + 4 + ia); k.ub0 = (s == 3) ? inf : __ldg(prm + 11 + ia);
-        k.lb1 = __ldg(prm + 4 + ib); k.ub1 = __ldg(prm + 11 + ib);
-        k.sl0 = k.cl0 = k.su0 = k.cu0 = 0.f;
-        float v_;
-        if (k.lb0 > -inf && k.ub0 < inf) { Num<float>::sincosv_(k.lb0, &k.sl0, &k.cl0, &v_); Num<float>::sincosv_(k.ub0, &k.su0, &k.cu0, &v_); }
+        const StageConst<float> k = stage_const(prm, s);
         // the seed enters like a carried angle: set_iterate + place, sin/cos derived from the placed value
-        float x0 = (s == 3) ? 0.f : place1(__ldg(prm + 18 + ia), k.lb0, k.ub0);
-        float x1 = place1(__ldg(prm + 18 + ib) - shift, k.lb1 - shift, k.ub1 - shift);
-        float sa = 0.f, ca = 1.f, sb, cb;
+        float x0 = (s == 3) ? 0.f : place1(__ldg(prm + 18 + k.ia), k.lb0, k.ub0);
+        float x1 = place1(__ldg(prm + 18 + k.ib) - k.shift, k.lb1s, k.ub1s);
+        float sa = 0.f, ca = 1.f, sb, cb, v_;
         if (s < 3) Num<float>::sincosv_(x0, &sa, &ca, &v_);
         Num<float>::sincosv_(x1, &sb, &cb, &v_);
         const Vec3<float> kt = map.apply({__ldg(kp + 3 * s + 3), __ldg(kp + 3 * s + 4), __ldg(kp + 3 * s + 5)}, s + 1);
         float xb; Vec3<float> w; uint32_t ne = 0u;
         serial_stage(s, k, a.gn_mask, esc, false, kt, o, A, piv, x0, x1, sa, ca, sb, cb, xb, w, ne, worst);
-        if (s < 3) ang[ia] = x0;
-        ang[ib] = xb;
-        if (kFk == 1) {
-            fk[3 * s] = o.x; fk[3 * s + 1] = o.y; fk[3 * s + 2] = o.z;
-            fk[15 + 3 * s] = w.x; fk[16 + 3 * s] = w.y; fk[17 + 3 * s] = w.z;
-            if (s == 0) { fk[12] = w.x; fk[13] = w.y; fk[14] = w.z; }
-        } else if (kFk == 2) { fk[3 * s] = w.x; fk[3 * s + 1] = w.y; fk[3 * s + 2] = w.z; }
+        if (s < 3) ang[k.ia] = x0;
+        ang[k.ib] = xb;
+        put_fk_joint<kFk>(fk, s, o, w);
         auto rec = [&](int i) -> float& { return ang[(int64_t)(1 + i / 7) * a.ang_fs + i % 7]; };
         rec(4 * s) = sa; rec(4 * s + 1) = ca; rec(4 * s + 2) = sb; rec(4 * s + 3) = cb;
         if (s < 3) rec(16 + s) = place1(x0, k.lb0, k.ub0);
-        rec(19 + s) = place1(x1, k.lb1 - shift, k.ub1 - shift);
+        rec(19 + s) = place1(x1, k.lb1s, k.ub1s);
         rec(23 + s) = __int_as_float((int)ne);
     }
     ang[(int64_t)4 * a.ang_fs + 6] = __int_as_float(worst);                  // record slot 27
@@ -467,18 +424,13 @@ leg_solve_block_kernel(LegArgs a, int bulk_in, int bulk_out, int first_done) {
     };
 
     if (lane < 4) {                                                // per-(chain, stage) constants
-        const int s = lane, ia = 2 * s, ib = (s == 3) ? 6 : 2 * s + 1;
-        const float shift = (s == 0) ? half_pi : 0.f;
-        const float lb0 = (s == 3) ? -inf : __ldg(BLK_PRM + 4 + ia), ub0 = (s == 3) ? inf : __ldg(BLK_PRM + 11 + ia);
-        const float lb1 = __ldg(BLK_PRM + 4 + ib), ub1 = __ldg(BLK_PRM + 11 + ib);
-        float* K = sh.kc[s];
-        K[KC_L] = __ldg(BLK_PRM + s); K[KC_LB0] = lb0; K[KC_UB0] = ub0; K[KC_LB1S] = lb1 - shift; K[KC_UB1S] = ub1 - shift;
-        K[KC_LB1] = lb1; K[KC_UB1] = ub1; K[KC_NSQ] = __ldg(BLK_PRM + 25 + s);
-        float sl = 0.f, cl = 0.f, su = 0.f, cu = 0.f, v_;
-        if (lb0 > -inf && ub0 < inf) { Num<float>::sincosv_(lb0, &sl, &cl, &v_); Num<float>::sincosv_(ub0, &su, &cu, &v_); }
-        K[KC_SL0] = sl; K[KC_CL0] = cl; K[KC_SU0] = su; K[KC_CU0] = cu;           // all zero: no limit case (warm_guess says interior)
-        K[KC_LB0P] = place1(lb0, lb0, ub0); K[KC_UB0P] = place1(ub0, lb0, ub0);
-        K[KC_HAVE_BT] = (s < 3 && cl * cl + sl * sl > 0.f) ? 1.f : 0.f;            // (the verification's have_bt, once per chain)
+        const StageConst<float> k = stage_const(BLK_PRM, lane);
+        float* K = sh.kc[lane];
+        K[KC_L] = k.L; K[KC_LB0] = k.lb0; K[KC_UB0] = k.ub0; K[KC_LB1S] = k.lb1s; K[KC_UB1S] = k.ub1s;
+        K[KC_LB1] = k.lb1; K[KC_UB1] = k.ub1; K[KC_NSQ] = k.nsq;
+        K[KC_SL0] = k.sl0; K[KC_CL0] = k.cl0; K[KC_SU0] = k.su0; K[KC_CU0] = k.cu0;
+        K[KC_LB0P] = k.lb0p; K[KC_UB0P] = k.ub0p;
+        K[KC_HAVE_BT] = (lane < 3 && k.cl0 * k.cl0 + k.sl0 * k.sl0 > 0.f) ? 1.f : 0.f;   // (the verification's have_bt, once per chain)
     }
     if (lane == 0) {
         mbar_init(&sh.bar[0], 1); mbar_init(&sh.bar[1], 1);
@@ -570,7 +522,7 @@ leg_solve_block_kernel(LegArgs a, int bulk_in, int bulk_out, int first_done) {
                         Tsa[s] = stash_f[9 * s]; Tca[s] = stash_f[9 * s + 1]; Tsb[s] = stash_f[9 * s + 2]; Tcb[s] = stash_f[9 * s + 3];
                         npv[s].x = stash_f[9 * s + 7]; npv[s].y = stash_f[9 * s + 8]; npv[s].z = stash_a[s < 3 ? s : 0];
                         if (s < 3) {
-                            A = rotate_frame(A, xy ? KIND_XY : KIND_ZY, Tsa[s], Tca[s], xy ? Tcb[s] : Tsb[s], xy ? -Tsb[s] : Tcb[s]);
+                            A = rotate_stage(A, s, Tsa[s], Tca[s], Tsb[s], Tcb[s]);
                             piv = npv[s];
                         }
                         continue;
@@ -655,7 +607,7 @@ leg_solve_block_kernel(LegArgs a, int bulk_in, int bulk_out, int first_done) {
                     const Vec3<float> np_ = {(piv.x + rel.x) + Af.x, (piv.y + rel.y) + Af.y, (piv.z + rel.z) + Af.z};
                     npv[s] = np_;
                     if (s < 3) {
-                        A = rotate_frame(A, xy ? KIND_XY : KIND_ZY, tsa, tca, xy ? tcb : tsb, xy ? -tsb : tcb);
+                        A = rotate_stage(A, s, tsa, tca, tsb, tcb);
                         piv = np_;
                     }
                 }
@@ -718,18 +670,8 @@ leg_solve_block_kernel(LegArgs a, int bulk_in, int bulk_out, int first_done) {
                 float* oa = sh.out_ang + lane * 7;
                 oa[0] = ox0[0]; oa[1] = ox1[0] + half_pi; oa[2] = ox0[1]; oa[3] = ox1[1]; oa[4] = ox0[2]; oa[5] = ox1[2]; oa[6] = ox1[3];
                 n_commit += 1u;
-                if (kFk == 1) {
-                    float* of = sh.out_fk + lane * 27;
 #pragma unroll
-                    for (int r = 0; r < 4; ++r) { of[3 * r] = o.x; of[3 * r + 1] = o.y; of[3 * r + 2] = o.z; }
-                    of[12] = npv[0].x + o.x; of[13] = npv[0].y + o.y; of[14] = npv[0].z + o.z;
-#pragma unroll
-                    for (int s = 0; s < 4; ++s) { of[15 + 3 * s] = npv[s].x + o.x; of[16 + 3 * s] = npv[s].y + o.y; of[17 + 3 * s] = npv[s].z + o.z; }
-                } else if (kFk == 2) {
-                    float* of = sh.out_fk + lane * 12;
-#pragma unroll
-                    for (int s = 0; s < 4; ++s) { of[3 * s] = npv[s].x + o.x; of[3 * s + 1] = npv[s].y + o.y; of[3 * s + 2] = npv[s].z + o.z; }
-                }
+                for (int s = 0; s < 4; ++s) put_fk_joint<kFk>(sh.out_fk + lane * FKF, s, o, {npv[s].x + o.x, npv[s].y + o.y, npv[s].z + o.z});
             }
             if (j >= nv) break;
             // ================= replay lane j through the serial solver, from its first failing stage =================
@@ -762,15 +704,9 @@ leg_solve_block_kernel(LegArgs a, int bulk_in, int bulk_out, int first_done) {
 #pragma unroll
                 for (int s = 0; s < 3; ++s) {
                     if (s < sf) {
-                        const bool xy = s == 0;
-                        oa[2 * s] = ox0[s]; oa[2 * s + 1] = xy ? ox1[s] + half_pi : ox1[s]; sh.nfx[s] += 1u;
-                        const Vec3<float> w = {npv[s].x + o.x, npv[s].y + o.y, npv[s].z + o.z};
-                        if (kFk == 1) {
-                            of[3 * s] = o.x; of[3 * s + 1] = o.y; of[3 * s + 2] = o.z;
-                            of[15 + 3 * s] = w.x; of[16 + 3 * s] = w.y; of[17 + 3 * s] = w.z;
-                            if (s == 0) { of[12] = w.x; of[13] = w.y; of[14] = w.z; }
-                        } else if (kFk == 2) { of[3 * s] = w.x; of[3 * s + 1] = w.y; of[3 * s + 2] = w.z; }
-                        A = rotate_frame(A, xy ? KIND_XY : KIND_ZY, Tsa[s], Tca[s], xy ? Tcb[s] : Tsb[s], xy ? -Tsb[s] : Tcb[s]);
+                        oa[2 * s] = ox0[s]; oa[2 * s + 1] = (s == 0) ? ox1[s] + half_pi : ox1[s]; sh.nfx[s] += 1u;
+                        put_fk_joint<kFk>(of, s, o, {npv[s].x + o.x, npv[s].y + o.y, npv[s].z + o.z});
+                        A = rotate_stage(A, s, Tsa[s], Tca[s], Tsb[s], Tcb[s]);
                         piv = npv[s];
                         sh.P[s][0] = Tsa[s]; sh.P[s][1] = Tca[s]; sh.P[s][2] = Tsb[s]; sh.P[s][3] = Tcb[s];
                     }
@@ -778,7 +714,7 @@ leg_solve_block_kernel(LegArgs a, int bulk_in, int bulk_out, int first_done) {
 #pragma unroll 1
                 for (int s = sf; s < 4; ++s) {
                     const float* K = sh.kc[s];
-                    const StageK k = {K[KC_L], K[KC_LB0], K[KC_UB0], K[KC_LB1], K[KC_UB1], K[KC_SL0], K[KC_CL0], K[KC_SU0], K[KC_CU0], K[KC_NSQ]};
+                    const SerialConst<float> k = {K[KC_L], K[KC_LB0], K[KC_UB0], K[KC_LB1], K[KC_UB1], K[KC_SL0], K[KC_CL0], K[KC_SU0], K[KC_CU0], K[KC_NSQ]};
                     float x0 = (s < 3) ? sh.acc_x[s < 3 ? s : 0][lane + 1] : 0.f, x1 = sh.acc_x[3 + s][lane + 1];
                     float sa = (s == 0) ? qsa[0] : (s == 1) ? qsa[1] : (s == 2) ? qsa[2] : qsa[3];
                     float ca = (s == 0) ? qca[0] : (s == 1) ? qca[1] : (s == 2) ? qca[2] : qca[3];
@@ -790,11 +726,7 @@ leg_solve_block_kernel(LegArgs a, int bulk_in, int bulk_out, int first_done) {
                     else serial_stage(s, k, a.gn_mask, esc, warm_ok, kt, o, A, piv, x0, x1, sa, ca, sb, cb, xb, w, ne, worst);
                     if (s < 3) { oa[2 * s] = x0; oa[2 * s + 1] = xb; } else oa[6] = xb;
                     sh.nfx[s] += ne;
-                    if (kFk == 1) {
-                        of[3 * s] = o.x; of[3 * s + 1] = o.y; of[3 * s + 2] = o.z;
-                        of[15 + 3 * s] = w.x; of[16 + 3 * s] = w.y; of[17 + 3 * s] = w.z;
-                        if (s == 0) { of[12] = w.x; of[13] = w.y; of[14] = w.z; }
-                    } else if (kFk == 2) { of[3 * s] = w.x; of[3 * s + 1] = w.y; of[3 * s + 2] = w.z; }
+                    put_fk_joint<kFk>(of, s, o, w);
                     // hand the final state on: the next pass starts from it
                     sh.P[s][0] = sa; sh.P[s][1] = ca; sh.P[s][2] = sb; sh.P[s][3] = cb;
                     // ... and the angles, as a reset of their series: x <- 0 x + (placed angle)

@@ -1,12 +1,11 @@
-// Host build of csrc/seqik_core.cuh for CPU-side algorithm tests (tests/ only).
+// Host build of csrc/seqik_core.cuh, seqik_generic.cuh and seqik_block.cuh for CPU-side algorithm tests (tests/ only).
+// The block schedule's emulation (run_block) runs the kernels' own replay and first-frame arithmetic (serial_stage).
 // TEST INFRASTRUCTURE: compiled by tests/hostsim_build.py with g++, loaded via ctypes by
 // tests; the product package never loads it.
 #include "seqik_core.cuh"
 #include "seqik_generic.cuh"
 #include "seqik_block.cuh"
 #include <cstdint>
-#include <cstdio>
-#include <cstdlib>
 
 using namespace seqik;
 
@@ -134,37 +133,21 @@ extern "C" void hostsim_carried_f32(const float* pose, int64_t n_frame, const fl
 // ---- the frame-parallel block schedule (csrc/seqik_block.cuh, leg_solve_block_kernel), emulated lane by lane: 32 frames of
 // a chain per pass (lane = frame, all four stages in the lane), closed-form candidates speculated from each frame's own key
 // points, angle increments accumulated in frame order, warm_step's admission tests verified with the exact angles, the first
-// lane that fails replayed through the serial solver.  Must equal run_carried bit for bit.
+// lane that fails replayed through the serial solver.  Must equal run_carried bit for bit.  The per-stage constants
+// (stage_const), the replay (serial_stage), the frame rotation and the forward-kinematics rows are the kernels' own code.
 // stats: [0] blocks, [1] passes, [2] serial frames, [3] serial frames by reason: first frame, [4] not admitted
-struct BlockStage {
-    int kind; bool xy, one_var; float L, has_a, shift, lb0, ub0, lb1, ub1, lb1s, ub1s, lb0p, ub0p, null_sq;
-    bool have_bt; float sl0, cl0, su0, cu0; int n_full, mode;
-};
 static void run_block(const float* pose, int64_t n_frame, const float* prm, const float* warm, float* angles, float* fk,
                       int32_t* nfev, int gn_mask, int64_t* stats) {
     typedef float R;
     const int W = 32;
-    const R inf = Num<R>::inf();
     const bool esc = (gn_mask >> 4) & 1;
-    BlockStage K[4];
-    for (int s = 0; s < 4; ++s) {
-        BlockStage& k = K[s];
-        const int ia = 2 * s, ib = (s == 3) ? 6 : 2 * s + 1;
-        k.kind = (s == 0) ? KIND_XY : KIND_ZY; k.xy = s == 0; k.one_var = s == 3;
-        k.L = prm[s]; k.has_a = (s == 3) ? 0.f : 1.f; k.shift = k.xy ? R(1.57079632679489661923) : R(0);
-        k.lb0 = (s == 3) ? -inf : prm[4 + ia]; k.ub0 = (s == 3) ? inf : prm[11 + ia];
-        k.lb1 = prm[4 + ib]; k.ub1 = prm[11 + ib]; k.lb1s = k.lb1 - k.shift; k.ub1s = k.ub1 - k.shift;
-        k.null_sq = prm[25 + s]; k.n_full = (s == 0) ? 4 : (s == 1) ? 6 : (s == 2) ? 8 : 9; k.mode = stage_mode(gn_mask, s);
-        k.have_bt = k.lb0 > -inf && k.ub0 < inf; k.sl0 = k.cl0 = k.su0 = k.cu0 = 0.f;
-        R v_;
-        if (k.have_bt) { Num<R>::sincosv_(k.lb0, &k.sl0, &k.cl0, &v_); Num<R>::sincosv_(k.ub0, &k.su0, &k.cu0, &v_); }
-        k.lb0p = place1(k.lb0, k.lb0, k.ub0); k.ub0p = place1(k.ub0, k.lb0, k.ub0);
-    }
+    StageConst<R> K[4];
+    for (int s = 0; s < 4; ++s) K[s] = stage_const(prm, s);
     // series l: 0..2 first angle of stages 1..3, 3..6 second angle of stages 1..4; carried in the caller's terms
     R xcar[7];
     const float* seed = warm ? warm : prm + 18;
-    for (int s = 0; s < 3; ++s) xcar[s] = seed[2 * s];
-    for (int s = 0; s < 4; ++s) xcar[3 + s] = seed[(s == 3) ? 6 : 2 * s + 1];
+    for (int s = 0; s < 3; ++s) xcar[s] = seed[K[s].ia];
+    for (int s = 0; s < 4; ++s) xcar[3 + s] = seed[K[s].ib];
     auto ser_lb = [&](int l) { return l < 3 ? K[l].lb0 : K[l - 3].lb1s; };
     auto ser_ub = [&](int l) { return l < 3 ? K[l].ub0 : K[l - 3].ub1s; };
     struct Trig { R sa, ca, sb, cb; };
@@ -199,7 +182,8 @@ static void run_block(const float* pose, int64_t n_frame, const float* prm, cons
                 const R* kp = pose + (t0 + t) * 15; org[t] = {kp[0], kp[1], kp[2]};
             }
             for (int s = 0; s < 4; ++s) {
-                const BlockStage& k = K[s];
+                const StageConst<R>& k = K[s];
+                const bool xy = s == 0, one_var = s == 3;
                 const R sgn = (P[s].sb < R(0)) ? R(-1) : R(1);
                 Vec3<R> res[W], rel[W];
                 for (int t = j0; t < nv; ++t) {
@@ -207,11 +191,11 @@ static void run_block(const float* pose, int64_t n_frame, const float* prm, cons
                     const Vec3<R> kt = {kp[3 * (s + 1)], kp[3 * (s + 1) + 1], kp[3 * (s + 1) + 2]};
                     rel[t] = {(kt.x - org[t].x) - piv[t].x, (kt.y - org[t].y) - piv[t].y, (kt.z - org[t].z) - piv[t].z};
                     const Vec3<R> q3 = mulT(A[t], rel[t]);
-                    const Vec3<R> q = k.xy ? Vec3<R>{-q3.z, q3.y, q3.x} : q3;
-                    const WarmCand<R> c = warm_interior(q, k.L, k.one_var, sgn, P[s].sa, P[s].ca);
+                    const Vec3<R> q = xy ? Vec3<R>{-q3.z, q3.y, q3.x} : q3;
+                    const WarmCand<R> c = warm_interior(q, k.L, one_var, sgn, P[s].sa, P[s].ca);
                     cond[s][t] = c.cond;
                     int g = WC_INTERIOR;
-                    if (k.have_bt && !k.one_var) g = warm_guess(c.n_sa, c.n_ca, k.sl0, k.cl0, k.su0, k.cu0);
+                    if (k.have_bt() && !one_var) g = warm_guess(c.n_sa, c.n_ca, k.sl0, k.cl0, k.su0, k.cu0);
                     guess[s][t] = g;
                     Vec3<R> f = c.f;
                     T[s][t] = {c.n_sa, c.n_ca, c.n_sb, c.n_cb};
@@ -226,7 +210,7 @@ static void run_block(const float* pose, int64_t n_frame, const float* prm, cons
                         outx0[s][t] = c.n_cb;
                         T[s][t] = {b_sa, b_ca, lc.c_sb, lc.c_cb};
                     }
-                    res[t] = k.xy ? Vec3<R>{f.z, f.y, -f.x} : f;
+                    res[t] = xy ? Vec3<R>{f.z, f.y, -f.x} : f;
                 }
                 for (int t = nv - 1; t >= j0; --t) {          // (descending: T[s][t-1] is read before lane t-1 parks anything)
                     const Trig pv = (t == j0) ? P[s] : T[s][t - 1];
@@ -244,8 +228,7 @@ static void run_block(const float* pose, int64_t n_frame, const float* prm, cons
                     const Vec3<R> Af = mul(A[t], res[t]);
                     const Vec3<R> np_ = {(piv[t].x + rel[t].x) + Af.x, (piv[t].y + rel[t].y) + Af.y, (piv[t].z + rel[t].z) + Af.z};
                     jw[s][t] = {np_.x + org[t].x, np_.y + org[t].y, np_.z + org[t].z};
-                    const R sin_b = k.xy ? T[s][t].cb : T[s][t].sb, cos_b = k.xy ? -T[s][t].sb : T[s][t].cb;
-                    A[t] = rotate_frame(A[t], k.kind, T[s][t].sa, T[s][t].ca, sin_b, cos_b);
+                    A[t] = rotate_stage(A[t], s, T[s][t].sa, T[s][t].ca, T[s][t].sb, T[s][t].cb);
                     piv[t] = np_;
                 }
             }
@@ -259,87 +242,51 @@ static void run_block(const float* pose, int64_t n_frame, const float* prm, cons
             for (int t = j0; t < nv && fail == nv; ++t) {
                 const bool enable_t = (t0 + t > 0) || warm != nullptr;
                 for (int s = 0; s < 4; ++s) {
-                    const BlockStage& k = K[s];
-                    const bool enable = enable_t && (k.mode & 8) && (k.mode & 1);
+                    const StageConst<R>& k = K[s];
+                    const int mode = stage_mode(gn_mask, s);
+                    const bool enable = enable_t && (mode & 8) && (mode & 1);
                     const R xp0 = (s < 3) ? acc_x[s][t] : R(0), xp1 = acc_x[3 + s][t];
                     WarmMove<R> mv; mv.dA = dA[s][t]; mv.dB = dB[s][t]; mv.small_a = sm_a[s][t]; mv.small_b = sm_b[s][t];
-                    const int wc = warm_case(enable, k.have_bt, k.one_var, xp0, xp1, mv, cond[s][t], k.lb0, k.ub0, k.lb1s, k.ub1s,
+                    const int wc = warm_case(enable, k.have_bt(), s == 3, xp0, xp1, mv, cond[s][t], k.lb0, k.ub0, k.lb1s, k.ub1s,
                                              guess[s][t], dB2[s][t], sm_b2[s][t], limq[s][t], outx0[s][t], outx1[s][t]);
-                    if (wc != guess[s][t]) {
-                        fail = t;
-                        if (getenv("HOSTSIM_BLOCK_LOG") && enable_t) {
-                            const R nx0 = xp0 + dA[s][t], nx1 = xp1 + dB[s][t];
-                            fprintf(stderr, "verify-fail frame %lld stage %d guess %d wc %d small_a %d small_b %d cond %d in_a %d in_b %d dA %.4g dB %.4g nx0 %.6g [%.6g %.6g] nx1 %.6g [%.6g %.6g] limq %d sm_b2 %d\n",
-                                    (long long)(t0 + t), s, guess[s][t], wc, (int)sm_a[s][t], (int)sm_b[s][t], (int)cond[s][t],
-                                    (int)((nx0 - k.lb0 > 1e-5f) & (k.ub0 - nx0 > 1e-5f)), (int)((nx1 - k.lb1s > 1e-5f) & (k.ub1s - nx1 > 1e-5f)),
-                                    (double)dA[s][t], (double)dB[s][t], (double)nx0, (double)k.lb0, (double)k.ub0, (double)nx1, (double)k.lb1s, (double)k.ub1s,
-                                    (int)limq[s][t], (int)sm_b2[s][t]);
-                        }
-                        break;
-                    }
+                    if (wc != guess[s][t]) { fail = t; break; }
                 }
             }
             // ---- commit lanes j0 .. fail-1
             for (int t = j0; t < fail; ++t) {
                 const int64_t ta = t0 + t;
                 for (int s = 0; s < 4; ++s) {
-                    if (s != 3) angles[ta * 7 + 2 * s] = outx0[s][t];
-                    angles[ta * 7 + ((s == 3) ? 6 : 2 * s + 1)] = outx1[s][t] + K[s].shift;
+                    if (s != 3) angles[ta * 7 + K[s].ia] = outx0[s][t];
+                    angles[ta * 7 + K[s].ib] = outx1[s][t] + K[s].shift;
                     nfev[ta * 4 + s] = 1;
-                    R* f9 = fk + ta * 27;
-                    f9[3 * s] = org[t].x; f9[3 * s + 1] = org[t].y; f9[3 * s + 2] = org[t].z;
-                    f9[15 + 3 * s] = jw[s][t].x; f9[16 + 3 * s] = jw[s][t].y; f9[17 + 3 * s] = jw[s][t].z;
-                    if (s == 0) { f9[12] = jw[s][t].x; f9[13] = jw[s][t].y; f9[14] = jw[s][t].z; }
+                    put_fk_joint<1>(fk + ta * 27, s, org[t], jw[s][t]);
                 }
             }
             if (fail == nv) break;
-            // ---- replay lane `fail` through the serial solver (run_carried's frame body), from the previous lane's state
+            // ---- replay lane `fail` through the serial solver, from the previous lane's state
             {
                 const int j = fail; const int64_t ta = t0 + j;
                 stats[2]++; stats[(ta == 0 && !warm) ? 3 : 4]++;
-                int n_seeded = 0;
                 const R* kp = pose + ta * 15;
                 const Vec3<R> o = {kp[0], kp[1], kp[2]};
                 Mat3<R> Aj = {{1.f, 0.f, 0.f}, {0.f, 1.f, 0.f}, {0.f, 0.f, 1.f}};
                 Vec3<R> pj = {0.f, 0.f, 0.f};
-                R* f9 = fk + ta * 27;
                 for (int s = 0; s < 4; ++s) {
-                    const BlockStage& k = K[s];
                     const Trig pv = (j == j0) ? P[s] : T[s][j - 1];
-                    StageSolve<R> S;
-                    S.set_problem(k.kind, k.L, k.has_a, k.null_sq, k.n_full, k.mode);
-                    S.have_bt = k.have_bt; S.sl0 = k.sl0; S.cl0 = k.cl0; S.su0 = k.su0; S.cu0 = k.cu0;
-                    S.x0 = (s < 3) ? acc_x[s][j] : R(0); S.x1 = acc_x[3 + s][j];
-                    S.sa = pv.sa; S.ca = pv.ca; S.sb = pv.sb; S.cb = pv.cb;
+                    R x0 = (s < 3) ? acc_x[s][j] : R(0), x1 = acc_x[3 + s][j];
+                    R sa = pv.sa, ca = pv.ca, sb = pv.sb, cb = pv.cb, xb;
                     const Vec3<R> kt = {kp[3 * (s + 1)], kp[3 * (s + 1) + 1], kp[3 * (s + 1) + 2]};
-                    const Vec3<R> rel = {(kt.x - o.x) - pj.x, (kt.y - o.y) - pj.y, (kt.z - o.z) - pj.z};
-                    const Vec3<R> q3 = mulT(Aj, rel);
-                    S.restart(q3, k.lb0, k.ub0, k.lb1, k.ub1, false, ta > 0 || warm != nullptr);
-                    for (;;) {
-                        while (!S.done()) S.trip();
-                        if (!(esc && S.escape())) break;
-                    }
-                    n_seeded += S.seeded && S.nfev == 1;
-                    if (getenv("HOSTSIM_BLOCK_LOG") && !(ta == 0 && !warm))
-                        fprintf(stderr, "replay frame %lld stage %d: seeded %d seed_at %d nfev %d status %d x0 %.7g lb0 %.7g ub0 %.7g x1 %.7g lb1s %.7g ub1s %.7g\n",
-                                (long long)ta, s, (int)S.seeded, S.seed_at, S.nfev, S.status, (double)S.x0, (double)k.lb0, (double)k.ub0, (double)S.x1, (double)k.lb1s, (double)k.ub1s);
-                    if (s != 3) angles[ta * 7 + 2 * s] = S.x0;
-                    angles[ta * 7 + ((s == 3) ? 6 : 2 * s + 1)] = S.angle_b();
-                    nfev[ta * 4 + s] = S.nfev;
-                    const Vec3<R> Af = mul(Aj, S.res());
-                    const Vec3<R> np_ = {(pj.x + rel.x) + Af.x, (pj.y + rel.y) + Af.y, (pj.z + rel.z) + Af.z};
-                    const Vec3<R> w = {np_.x + o.x, np_.y + o.y, np_.z + o.z};
-                    f9[3 * s] = o.x; f9[3 * s + 1] = o.y; f9[3 * s + 2] = o.z;
-                    f9[15 + 3 * s] = w.x; f9[16 + 3 * s] = w.y; f9[17 + 3 * s] = w.z;
-                    if (s == 0) { f9[12] = w.x; f9[13] = w.y; f9[14] = w.z; }
-                    Aj = rotate_frame(Aj, k.kind, S.sa, S.ca, S.sin_b(), S.cos_b());
-                    pj = np_;
-                    T[s][j] = {S.sa, S.ca, S.sb, S.cb};
-                    if (s < 3) acc_x[s][j + 1] = place1(S.x0, k.lb0, k.ub0);
-                    acc_x[3 + s][j + 1] = place1(S.x1, k.lb1s, k.ub1s);
+                    Vec3<R> w; uint32_t ne = 0u; int worst = ST_GTOL;
+                    serial_stage(s, K[s], gn_mask, esc, ta > 0 || warm != nullptr, kt, o, Aj, pj, x0, x1, sa, ca, sb, cb, xb, w, ne, worst);
+                    if (s != 3) angles[ta * 7 + K[s].ia] = x0;
+                    angles[ta * 7 + K[s].ib] = xb;
+                    nfev[ta * 4 + s] = (int32_t)ne;
+                    put_fk_joint<1>(fk + ta * 27, s, o, w);
+                    T[s][j] = {sa, ca, sb, cb};
+                    if (s < 3) acc_x[s][j + 1] = place1(x0, K[s].lb0, K[s].ub0);
+                    acc_x[3 + s][j + 1] = place1(x1, K[s].lb1s, K[s].ub1s);
                 }
                 for (int s = 0; s < 4; ++s) P[s] = T[s][j];
-                if (n_seeded == 4) stats[5]++;
                 j0 = j + 1;
                 if (j0 >= nv) break;
             }

@@ -96,7 +96,7 @@ def run_block_f32(pose, prm, gn_mask=0xFF, warm=None):
     angles = np.zeros((n, 7), dtype=np.float32)
     fk = np.zeros((n, 9, 3), dtype=np.float32)
     nfev = np.zeros((n, 4), dtype=np.int32)
-    stats = np.zeros(8, dtype=np.int64)
+    stats = np.zeros(5, dtype=np.int64)
     w = None if warm is None else np.ascontiguousarray(warm, dtype=np.float32)
     P = ctypes.c_void_p
     fn = lib.hostsim_block_f32
