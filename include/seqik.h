@@ -195,7 +195,9 @@ int seqik_fk_f32(const float* angles, const float* origin, int64_t origin_frame_
  *   affine_r, affine_l: NULL, or [n_trial][8] head-alignment rows (see seqik_head_affine_f32) applied on load
  *   rest [n_trial][2] = (rest_head_pitch, rest_antenna_pitch) (head_inverse_kinematics.py:309-329)
  *   out [n_trial][7][n_frame]: head_roll, head_pitch, head_yaw, antenna_yaw_L, antenna_pitch_L,
- *   antenna_yaw_R, antenna_pitch_R */
+ *   antenna_yaw_R, antenna_pitch_R
+ * Any 4-byte aligned r_head / l_head works: 8-byte aligned inputs are read with 64-bit loads, others (e.g. a view at an odd
+ * float offset) with 32-bit loads, with bit-identical results. */
 int seqik_head_angles_f32(const float* r_head, const float* l_head, const float* neck, int64_t neck_stride,
                           const float* affine_r, const float* affine_l, const float* rest,
                           float* out, int64_t n_trial, int64_t n_frame, void* stream);

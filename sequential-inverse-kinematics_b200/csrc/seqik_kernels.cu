@@ -328,8 +328,9 @@ extern "C" int seqik_fk_f32(const float* angles, const float* origin, int64_t or
 // angle_between_segments (head_inverse_kinematics.py:163-183) for vectors that live in a coordinate plane:
 // arccos(v1^.v2^) * (det > 0 ? 1 : -1), evaluated as atan2(|det|, dot) which keeps FP32 accuracy near 0 and pi.
 // atan2(y, x) for y >= 0, result in [0, pi]: octant reduction to t = min/max in [0, 1], one more reduction at tan(pi/8)
-// ((t - 1) / (t + 1)), then the degree-4 minimax polynomial in t^2 of Cephes' atanf (|error| < 2e-7 rad including the two
-// SFU reciprocals; the parity bound of the head angles is 2e-5 rad).  Half the instructions of atan2f, no slow path:
+// ((t - 1) / (t + 1)), then the degree-4 minimax polynomial in t^2 of Cephes' atanf (|error| < half an ulp of the result
+// + 2e-7 rad including the two SFU reciprocals, i.e. < 3.2e-7 rad near pi, tests/test_gpu_stream.py; the parity bound of
+// the head angles is 2e-5 rad).  Half the instructions of atan2f, no slow path:
 // the head kernel is issue-bound on its five arctangents per frame.
 __device__ __forceinline__ float atan2_pos(float y, float x) {
     const float ax = fabsf(x);
@@ -397,6 +398,9 @@ __device__ __forceinline__ void head_frame(const float* rr, const float* ll, con
     }
 }
 
+// kVec2: r_head and l_head are 8-byte aligned and read as 64-bit loads; otherwise (a view at an odd float offset) the same
+// six floats are read one by one -- the arithmetic, hence the result, is the same
+template <bool kVec2>
 __global__ void __launch_bounds__(256) head_kernel(const float* __restrict__ r_head, const float* __restrict__ l_head,
                                                    const float* __restrict__ neck, int64_t neck_stride,
                                                    const float* __restrict__ affine_r, const float* __restrict__ affine_l,
@@ -406,11 +410,18 @@ __global__ void __launch_bounds__(256) head_kernel(const float* __restrict__ r_h
     if (i >= n_trial * n_frame) return;
     const int64_t tr = i / n_frame, t = i - tr * n_frame;
     const float* r = r_head + i * 6; const float* l = l_head + i * 6;        // 24-byte records: three 64-bit loads each
-    const float2 r01 = __ldg(reinterpret_cast<const float2*>(r)), r23 = __ldg(reinterpret_cast<const float2*>(r) + 1),
-                 r45 = __ldg(reinterpret_cast<const float2*>(r) + 2);
-    const float2 l01 = __ldg(reinterpret_cast<const float2*>(l)), l23 = __ldg(reinterpret_cast<const float2*>(l) + 1),
-                 l45 = __ldg(reinterpret_cast<const float2*>(l) + 2);
-    const float rr[6] = {r01.x, r01.y, r23.x, r23.y, r45.x, r45.y}, ll[6] = {l01.x, l01.y, l23.x, l23.y, l45.x, l45.y};
+    float rr[6], ll[6];
+    if (kVec2) {
+        const float2 r01 = __ldg(reinterpret_cast<const float2*>(r)), r23 = __ldg(reinterpret_cast<const float2*>(r) + 1),
+                     r45 = __ldg(reinterpret_cast<const float2*>(r) + 2);
+        const float2 l01 = __ldg(reinterpret_cast<const float2*>(l)), l23 = __ldg(reinterpret_cast<const float2*>(l) + 1),
+                     l45 = __ldg(reinterpret_cast<const float2*>(l) + 2);
+        rr[0] = r01.x; rr[1] = r01.y; rr[2] = r23.x; rr[3] = r23.y; rr[4] = r45.x; rr[5] = r45.y;
+        ll[0] = l01.x; ll[1] = l01.y; ll[2] = l23.x; ll[3] = l23.y; ll[4] = l45.x; ll[5] = l45.y;
+    } else {
+#pragma unroll
+        for (int k = 0; k < 6; ++k) { rr[k] = __ldg(r + k); ll[k] = __ldg(l + k); }
+    }
     float o7[7];
     head_frame(rr, ll, neck + (neck_stride ? i * 3 : tr * 3), affine_r ? affine_r + tr * 8 : nullptr,
                affine_l ? affine_l + tr * 8 : nullptr, rest[tr * 2], rest[tr * 2 + 1], o7);
@@ -431,8 +442,11 @@ extern "C" int seqik_head_angles_f32(const float* r_head, const float* l_head, c
     const int64_t n = n_trial * n_frame;
     // (stays on plain loads: five atan2f and a sincos per 76-byte frame make this kernel issue-bound at ~0.57 of the HBM
     // peak with 2048 threads per SM; the 1024-thread TMA pipeline measured slower here, 0.37)
-    head_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(r_head, l_head, neck, neck_stride, affine_r, affine_l,
-                                                                              rest, out, n_trial, n_frame);
+    // any 4-byte aligned head input is accepted: a view at an odd float offset takes the scalar-load instantiation
+    const bool vec2 = ((((uintptr_t)r_head) | ((uintptr_t)l_head)) & 7) == 0;
+    auto kernel = vec2 ? head_kernel<true> : head_kernel<false>;
+    kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(r_head, l_head, neck, neck_stride, affine_r, affine_l,
+                                                                         rest, out, n_trial, n_frame);
     return check_launch("seqik_head_angles_f32");
 }
 
