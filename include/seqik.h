@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define SEQIK_ABI_VERSION 8   /* 8: seqik_origin_rows_f32; 7: seqik_leg_affine_from_pose_f32; 6: schedule 3 (frame-parallel blocks), seqik_fk_expand_host_f32; 5: solver flag bits 6-7, phase periods in bits 21-27 */
+#define SEQIK_ABI_VERSION 9   /* 9: seqik_fk_backward_f32; 8: seqik_origin_rows_f32; 7: seqik_leg_affine_from_pose_f32; 6: schedule 3 (frame-parallel blocks), seqik_fk_expand_host_f32; 5: solver flag bits 6-7, phase periods in bits 21-27 */
 #define SEQIK_OK 0
 #define SEQIK_EINVAL (-1)
 #define SEQIK_ECUDA (-3)
@@ -187,6 +187,25 @@ int seqik_leg_solve_generic_f64(const double* pose, int64_t pose_chain_stride, i
  *   origin_frame_stride = 0), params as above, fk [n_chain][n_frame][9][3]; all dense. */
 int seqik_fk_f32(const float* angles, const float* origin, int64_t origin_frame_stride, const float* params,
                  float* fk, int64_t n_chain, int64_t n_frame, void* stream);
+
+/* Backward of seqik_fk_f32 (vector-Jacobian product): the gradient of a loss L with respect to the angles, the origin and
+ * the segment lengths, given grad_fk = dL/dfk.  New in this library: the reference has no gradients, so this replaces
+ * nothing in it.
+ *   angles, origin, origin_frame_stride, params: as for seqik_fk_f32 (params[0..3] are the only entries FK reads).  The
+ *   gradients do not depend on the origin (FK is a translation by it): it is checked for NULL but not read.
+ *   grad_fk      [n_chain][n_frame][9][3] in
+ *   grad_angles  [n_chain][n_frame][7] out (required)
+ *   grad_origin  NULL (skip), or [n_chain][n_frame][3] out: dL/dorigin PER FRAME, also when origin_frame_stride = 0 (the
+ *                caller sums over frames).  Per coordinate, in float32 and in this order (g_r = row r of grad_fk):
+ *                  S4 = g8;  S3 = g7 + S4;  S2 = g6 + S3;  S1 = (g4 + g5) + S2;
+ *                  grad_origin = (((g0 + g1) + g2) + g3) + S1
+ *   grad_lengths NULL (skip), or [n_chain][n_frame][4] out: per-frame contributions to dL/dparams[0..3] (the caller sums
+ *                over frames; no other params entry has a gradient)
+ * All arrays dense.  The forward is recomputed with the arithmetic of seqik_fk_f32; results are deterministic (no
+ * atomics) and do not depend on the launch path. */
+int seqik_fk_backward_f32(const float* angles, const float* origin, int64_t origin_frame_stride, const float* params,
+                          const float* grad_fk, float* grad_angles, float* grad_origin, float* grad_lengths,
+                          int64_t n_chain, int64_t n_frame, void* stream);
 
 /* Head roll/pitch/yaw and antenna yaw/pitch (L then R).
  * Replaces HeadInverseKinematics.compute_head_angles (seqikpy/head_inverse_kinematics.py:103-142, 163-307).

@@ -1,6 +1,7 @@
 """HBM-bound satellite kernels against the measured copy bandwidth (GPU box).  Prints one JSON line per kernel.
 
-Algorithmic bytes per unit (DESIGN.md 5.3): fk 28+12+108 B/leg-frame (origin per frame), head 48+28 B/frame (+12 with a
+Algorithmic bytes per unit (DESIGN.md 5.3): fk 28+12+108 B/leg-frame (origin per frame), fk backward 28+108 in and 28+12
+(+16 with the lengths) out, head 48+28 B/frame (+12 with a
 per-frame neck), align_apply 60+60 B/leg-frame, leg_series 60 in + 28 out, mid_quantile 4 B/element read (4 ranks x
 4 radix passes re-read the series: from L2 when it fits)."""
 import json, sys
@@ -45,6 +46,25 @@ angles += 0.01 * torch.randn(angles.shape, device="cuda", generator=g)
 origin = torch.randn((n_chain, n_frame, 3), device="cuda", generator=g)
 lf = n_chain * n_frame
 report("fk_kernel", timeit(lambda: engine.forward_kinematics(angles, origin, params)), lf * (28 + 12 + 108), lf, "leg-frames")
+# FK backward: angles + grad_fk in (the origin is not read: FK is a translation by it), grad_angles + grad_origin out (+ grad_lengths)
+grad_fk = torch.randn((n_chain, n_frame, 9, 3), device="cuda", generator=g)
+report("fk_backward_kernel", timeit(lambda: engine.forward_kinematics_backward(angles, origin, params, grad_fk)),
+       lf * (28 + 108 + 28 + 12), lf, "leg-frames")
+report("fk_backward_kernel, with grad_lengths", timeit(lambda: engine.forward_kinematics_backward(angles, origin, params, grad_fk, want_lengths=True)),
+       lf * (28 + 108 + 28 + 12 + 16), lf, "leg-frames")
+# forward + VJP (angles, origin): through engine.forward_kinematics' autograd, and through torch autograd of the same FK in
+# float32 torch ops (tests/model_fk.py: what a user writes without the kernel).  Bytes: those of the two kernels.
+sys.path.insert(0, str(ROOT / "tests"))
+import model_fk
+a_req, o_req = angles.clone().requires_grad_(), origin.clone().requires_grad_()
+lengths = params[:, None, :4]
+report("forward_kinematics + backward through autograd (kernels)",
+       timeit(lambda: torch.autograd.grad(engine.forward_kinematics(a_req, o_req, params), [a_req, o_req], grad_fk)),
+       lf * (28 + 12 + 108 + 28 + 108 + 28 + 12), lf, "leg-frames")
+report("float32 torch-ops FK + torch autograd VJP (reference point)",
+       timeit(lambda: torch.autograd.grad(model_fk.fk(a_req, o_req, lengths), [a_req, o_req], grad_fk), reps=3),
+       lf * (28 + 12 + 108 + 28 + 108 + 28 + 12), lf, "leg-frames")
+del grad_fk, a_req, o_req
 pose = torch.randn((n_chain, n_frame, 5, 3), device="cuda", generator=g)
 aff = torch.rand((n_chain, 8), device="cuda", generator=g) + 0.5
 report("align_apply_kernel", timeit(lambda: engine.align_apply(pose, aff)), lf * 120, lf, "leg-frames")

@@ -161,26 +161,101 @@ def leg_solve_generic(pose, params, target_row: int = -1, want_fk: bool = True, 
     return angles, fk, status, nfev
 
 
-def forward_kinematics(angles, origin, params):
-    """angles (n_chain, n_frame, 7) + origin (n_chain, n_frame, 3) or (n_chain, 3) -> fk (n_chain, n_frame, 9, 3)."""
-    torch = N.require_cuda()
-    lib = N.load_library()
+def _fk_inputs(angles, origin, params):
+    """Checks of the FK inputs -> (n_chain, n_frame, origin frame stride)."""
     angles = _check(angles, "angles", (7,))
     n_chain, n_frame = int(angles.shape[0]), int(angles.shape[1])
     origin = _check(origin, "origin", (3,))
     params = _check(params, "params", (N.CHAIN_PARAM_FLOATS,))
     if origin.dim() == 3 and tuple(origin.shape[:2]) == (n_chain, n_frame):
-        stride = 3
-    elif origin.dim() == 2 and origin.shape[0] == n_chain:
-        stride = 0
-    else:
-        raise ValueError("origin must be (n_chain, n_frame, 3) or (n_chain, 3)")
+        return n_chain, n_frame, 3
+    if origin.dim() == 2 and origin.shape[0] == n_chain:
+        return n_chain, n_frame, 0
+    raise ValueError("origin must be (n_chain, n_frame, 3) or (n_chain, 3)")
+
+
+def forward_kinematics(angles, origin, params):
+    """angles (n_chain, n_frame, 7) + origin (n_chain, n_frame, 3) or (n_chain, 3) -> fk (n_chain, n_frame, 9, 3).
+
+    Differentiable: when grad mode is on and any input requires grad, the result carries a ``grad_fn`` whose backward is
+    the ``seqik_fk_backward_f32`` kernel (see ``forward_kinematics_backward``).  ``params`` then gets an (n_chain, 32)
+    gradient with the segment lengths' gradients in columns 0-3 and zeros elsewhere (no other entry enters FK); an
+    (n_chain, 3) origin gets the sum over frames.  First derivatives only: a second backward raises.  Without inputs that
+    require grad the call is the plain kernel launch."""
+    torch = N.require_cuda()
+    if torch.is_grad_enabled() and any(isinstance(t, torch.Tensor) and t.requires_grad for t in (angles, origin, params)):
+        return _fk_function().apply(angles, origin, params)
+    return _forward_kinematics(torch, angles, origin, params)
+
+
+def _forward_kinematics(torch, angles, origin, params):
+    lib = N.load_library()
+    n_chain, n_frame, stride = _fk_inputs(angles, origin, params)
     fk = torch.empty((n_chain, n_frame, 9, 3), dtype=torch.float32, device=angles.device)
     with torch.cuda.device(angles.device):
         rc = lib.seqik_fk_f32(N.ptr(angles), N.ptr(origin), stride, N.ptr(params), N.ptr(fk), n_chain, n_frame,
                               N.stream_ptr(torch, angles.device))
     N.check(rc, "seqik_fk_f32")
     return fk
+
+
+def forward_kinematics_backward(angles, origin, params, grad_fk, want_origin: bool = True, want_lengths: bool = False):
+    """Vector-Jacobian product of ``forward_kinematics``: grad_fk (n_chain, n_frame, 9, 3) = dL/dfk ->
+    (grad_angles (n_chain, n_frame, 7), grad_origin (n_chain, n_frame, 3) | None, grad_lengths (n_chain, n_frame, 4) | None),
+    all per leg-frame: grad_origin is per frame also for an (n_chain, 3) origin, and grad_lengths holds each frame's
+    contribution to dL/dparams[:, 0:4].  Sum over frames where the input is shared.  The summation order of grad_origin is
+    that of include/seqik.h."""
+    torch = N.require_cuda()
+    lib = N.load_library()
+    n_chain, n_frame, stride = _fk_inputs(angles, origin, params)
+    grad_fk = _check(grad_fk, "grad_fk", (9, 3))
+    if tuple(grad_fk.shape) != (n_chain, n_frame, 9, 3):
+        raise ValueError(f"grad_fk must be ({n_chain}, {n_frame}, 9, 3), got {tuple(grad_fk.shape)}")
+    dev = angles.device
+    grad_angles = torch.empty((n_chain, n_frame, 7), dtype=torch.float32, device=dev)
+    grad_origin = torch.empty((n_chain, n_frame, 3), dtype=torch.float32, device=dev) if want_origin else None
+    grad_lengths = torch.empty((n_chain, n_frame, 4), dtype=torch.float32, device=dev) if want_lengths else None
+    with torch.cuda.device(dev):
+        rc = lib.seqik_fk_backward_f32(N.ptr(angles), N.ptr(origin), stride, N.ptr(params), N.ptr(grad_fk), N.ptr(grad_angles),
+                                       N.ptr(grad_origin), N.ptr(grad_lengths), n_chain, n_frame, N.stream_ptr(torch, dev))
+    N.check(rc, "seqik_fk_backward_f32")
+    return grad_angles, grad_origin, grad_lengths
+
+
+_FK_FUNCTION = None
+
+
+def _fk_function():
+    """The torch.autograd.Function of forward_kinematics (built on first use: torch is imported lazily)."""
+    global _FK_FUNCTION
+    if _FK_FUNCTION is not None:
+        return _FK_FUNCTION
+    import torch
+    from torch.autograd.function import once_differentiable
+
+    class ForwardKinematics(torch.autograd.Function):
+        @staticmethod
+        def forward(ctx, angles, origin, params):
+            ctx.save_for_backward(angles, origin, params)
+            return _forward_kinematics(torch, angles, origin, params)
+
+        @staticmethod
+        @once_differentiable
+        def backward(ctx, grad_fk):
+            angles, origin, params = ctx.saved_tensors
+            need_angles, need_origin, need_params = ctx.needs_input_grad
+            ga, go, gl = forward_kinematics_backward(angles, origin, params, grad_fk.contiguous(),
+                                                     want_origin=need_origin, want_lengths=need_params)
+            if need_origin and origin.dim() == 2:
+                go = go.sum(dim=1)
+            g_params = None
+            if need_params:
+                g_params = torch.zeros_like(params)
+                g_params[:, :4] = gl.sum(dim=1)
+            return (ga if need_angles else None), go, g_params
+
+    _FK_FUNCTION = ForwardKinematics
+    return _FK_FUNCTION
 
 
 def head_angles(r_head, l_head, neck, rest, affine_r=None, affine_l=None):
