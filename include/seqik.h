@@ -226,7 +226,11 @@ int seqik_head_angles_f32(const float* r_head, const float* l_head, const float*
  * (seqikpy/alignment.py:83-87, 392-415).
  *   series [n_series][n] (dense rows); counts NULL, or [n_series] int32: only the counts[i] SMALLEST values of
  *   row i take part (rows padded with +inf, see seqik_head_series_f32); out [n_series];
- *   scratch: unused (may be NULL); kept so that the signature is stable */
+ *   scratch: unused (may be NULL); kept so that the signature is stable
+ * Values are ordered by their bits: -0 sorts below +0, a NaN with the sign bit clear above +inf and one with the sign
+ * bit set below -inf; a NaN among the four order statistics makes the result NaN.  The four order statistics are
+ * exact; each quantile is a + (b - a) f in float32 with f = float32(q (m - 1) - floor(q (m - 1))), m the values taking
+ * part, and out = 0.5f (q45 + q55).  counts[i] <= 0 gives NaN; counts[i] > n is outside the contract. */
 int seqik_mid_quantile_f32(const float* series, const int32_t* counts, float* scratch, float* out,
                            int64_t n_series, int64_t n, void* stream);
 

@@ -402,7 +402,11 @@ extern "C" int seqik_leg_series_f32(const float* pose, int64_t pose_chain_stride
 
 // Order statistic by 4-pass MSB radix select on order-preserving keys; one block per (series, rank).
 __device__ __forceinline__ uint32_t order_key(float f) {
-    const uint32_t u = __float_as_uint(f);
+    // The bits go through an opaque move.  From __float_as_uint(f), the compiler turned `u | 0x80000000` into a float
+    // negation of |f| (FADD -|f|, -0), which makes a NaN the canonical 0x7fffffff: a key just below +0's, inside any range
+    // that straddles zero (the long kernel's NaN padding of its float4 sweeps included).
+    uint32_t u;
+    asm("mov.b32 %0, %1;" : "=r"(u) : "f"(f));
     return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
 }
 __device__ __forceinline__ float key_value(uint32_t k) {
@@ -505,7 +509,8 @@ __global__ void __launch_bounds__(SEL_BLOCK) mid_quantile_kernel(const float* __
 //     per rank): the next pass sweeps those only, and with 32 or fewer left the ranks are read off directly (each lane counts
 //     the keys below its own);
 //   * packs the four histograms into 256 words of two 16-bit pairs (counts <= 1024): 2 KB per warp.
-// Bit-compatible with np.quantile(..., method="linear") on float32 input, like the kernel it replaces.
+// The order statistics are exact; the interpolation (mid_quantile_value) is a + (b - a) f in float32, like the kernel it
+// replaces -- within 2 u |q| of np.quantile(..., method="linear") in float64 for same-sign statistics, not always its bits.
 constexpr int WQ_N = 1024, WQ_WARPS = 4;
 __device__ __forceinline__ uint32_t low_mask(int nb) { return nb >= 32 ? 0xffffffffu : ((1u << nb) - 1u); }
 
@@ -664,24 +669,30 @@ __device__ void warp_select4(uint32_t* __restrict__ key, int n, unsigned int* ra
     }
 }
 
-// the four ranks of the mid-quantile of the m smallest keys, and the interpolation weights (numpy "linear")
-__device__ __forceinline__ void mid_quantile_ranks(int64_t m, unsigned int* rank, float& f45, float& f55) {
+// the four ranks of the mid-quantile of the m smallest keys, and the interpolation weights (numpy "linear").  The ranks
+// come out non-decreasing, as warp_select4 and the long kernel's bin search require: for m = 2, 4, 6, 8, 10 both positions
+// have the same lower neighbour (lo45 == lo55), and lo, lo + 1, lo, lo + 1 is selected as lo, lo, lo + 1, lo + 1.  The
+// return value says so; mid_quantile_value puts the middle two back.
+__device__ __forceinline__ bool mid_quantile_ranks(int64_t m, unsigned int* rank, float& f45, float& f55) {
     int64_t lo45, lo55;
     quantile_pos(0.45, m, lo45, f45); quantile_pos(0.55, m, lo55, f55);
 #pragma unroll
     for (int k = 0; k < 4; ++k) { const int64_t r = (k < 2 ? lo45 : lo55) + (k & 1); rank[k] = (unsigned int)(r > m - 1 ? m - 1 : r); }
+    const bool swap = rank[1] > rank[2];
+    if (swap) { const unsigned int t = rank[1]; rank[1] = rank[2]; rank[2] = t; }
+    return swap;
 }
-__device__ __forceinline__ float mid_quantile_value(const uint32_t* val, float f45, float f55) {
-    const float a0 = key_value(val[0]), a1 = key_value(val[1]), b0 = key_value(val[2]), b1 = key_value(val[3]);
+__device__ __forceinline__ float mid_quantile_value(const uint32_t* val, float f45, float f55, bool swap) {
+    const float a0 = key_value(val[0]), a1 = key_value(val[swap ? 2 : 1]), b0 = key_value(val[swap ? 1 : 2]), b1 = key_value(val[3]);
     const float q0 = a0 + (a1 - a0) * f45, q1 = b0 + (b1 - b0) * f55;
     return 0.5f * (q0 + q1);
 }
 // key[0..n): order keys of the series (shared memory, 16-byte aligned, overwritten); m: the m smallest take part
 __device__ float warp_mid_quantile(uint32_t* __restrict__ key, int n, int64_t m, unsigned int (*hist)[256], int lane) {
     unsigned int rank[4]; uint32_t val[4]; float f45, f55;
-    mid_quantile_ranks(m, rank, f45, f55);
+    const bool swap = mid_quantile_ranks(m, rank, f45, f55);
     warp_select4(key, n, rank, hist, lane, val);
-    return mid_quantile_value(val, f45, f55);
+    return mid_quantile_value(val, f45, f55, swap);
 }
 
 __global__ void __launch_bounds__(32 * WQ_WARPS) mid_quantile_warp_kernel(const float* __restrict__ series, const int32_t* __restrict__ counts,
@@ -757,12 +768,13 @@ __global__ void __launch_bounds__(LA_THREADS) leg_affine_fused_kernel(const floa
     }
     {
         unsigned int rank[4]; uint32_t val[4]; float f45, f55;
-        mid_quantile_ranks(n_frame, rank, f45, f55);
+        const bool swap = mid_quantile_ranks(n_frame, rank, f45, f55);
         warp_select4(key[w], n_frame, rank, u.hist[w], lane, val);
         if (lane == 0) {
             float v4[4];
 #pragma unroll
             for (int t = 0; t < 4; ++t) { v4[t] = key_value(val[t]); if (w >= 3) v4[t] = sqrtf(v4[t]); }
+            if (swap) { const float t = v4[1]; v4[1] = v4[2]; v4[2] = t; }
             const float q0 = v4[0] + (v4[1] - v4[0]) * f45, q1 = v4[2] + (v4[3] - v4[2]) * f55;
             stat[w] = 0.5f * (q0 + q1);
         }
@@ -801,13 +813,13 @@ __global__ void __launch_bounds__(LQ_BLOCK) mid_quantile_long_kernel(const float
     const int64_t m = counts ? (int64_t)counts[sidx] : n;
     if (m <= 0) { if (tid == 0) out[sidx] = __int_as_float(0x7fc00000); return; }
     unsigned int rank[4]; uint32_t val[4]; float f45, f55;
-    mid_quantile_ranks(m, rank, f45, f55);
+    const bool swap = mid_quantile_ranks(m, rank, f45, f55);
     if (n <= LQ_CAND) {
         for (int i = tid; i < (int)n; i += LQ_BLOCK) cand[i] = order_key(__ldg(v + i));
         __syncthreads();
         if (w == 0) {
             warp_select4(cand, (int)n, rank, reinterpret_cast<unsigned int (*)[256]>(hist), lane, val);
-            if (lane == 0) out[sidx] = mid_quantile_value(val, f45, f55);
+            if (lane == 0) out[sidx] = mid_quantile_value(val, f45, f55, swap);
         }
         return;
     }
@@ -907,7 +919,7 @@ __global__ void __launch_bounds__(LQ_BLOCK) mid_quantile_long_kernel(const float
         // the range spans fewer than 4096 distinct keys (a constant or few-valued series): a bin IS a key value
         if (tid == 0) {
             val[0] = smin + (uint32_t)b0; val[1] = smin + (uint32_t)b1; val[2] = smin + (uint32_t)b2; val[3] = smin + (uint32_t)b3;
-            out[sidx] = mid_quantile_value(val, f45, f55);
+            out[sidx] = mid_quantile_value(val, f45, f55, swap);
         }
         return;
     }
@@ -939,7 +951,7 @@ __global__ void __launch_bounds__(LQ_BLOCK) mid_quantile_long_kernel(const float
     __syncthreads();
     if (w == 0) {
         warp_select4(cand, (int)c, lrank, reinterpret_cast<unsigned int (*)[256]>(hist), lane, val);
-        if (lane == 0) out[sidx] = mid_quantile_value(val, f45, f55);
+        if (lane == 0) out[sidx] = mid_quantile_value(val, f45, f55, swap);
     }
 }
 

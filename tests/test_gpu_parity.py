@@ -498,8 +498,8 @@ def test_mid_quantile_narrow_ranges_ties_and_counts(api):
     t = api.torch
     rng = np.random.default_rng(11)
     for n in (1, 2, 31, 32, 33, 64, 65, 500, 1000, 1023, 1024, 1025, 4096, 4097, 20000, 100003):
-        # (beyond 1024 samples: the sampled-range two-sweep kernel; the two-valued and the four-valued series have more
-        #  candidates than it keeps and go through the general kernel, the drifting one has its ranks inside the sample's range)
+        # (beyond 4096 samples: the sampled-range kernel; the constant, two-valued and four-valued series span fewer than
+        #  4096 keys and are read off its first sweep's histogram (shift 0); tests/test_gpu_quantile.py covers every route)
         rows = [0.7312 + 1e-3 * rng.normal(size=n), np.full(n, -3.25), rng.choice([1.5, 1.5000001], size=n),
                 1e-3 * rng.normal(size=n), np.where(rng.random(n) < 0.5, 0.0, -0.0), 1e30 * rng.normal(size=n),
                 np.sort(rng.normal(size=n)), 0.4 + 1e-6 * rng.integers(0, 4, size=n),
