@@ -186,6 +186,13 @@ enum : int {
     ST_NONFINITE = -2      // residual not finite at the start of a solve (scipy raises there): the solve is skipped
 };
 
+// An angle is written out clamped to its limits.  The iterate itself can sit one float32 ulp (or, on a limit at 0, one
+// FLT_MIN) outside the box: the bound distances are carried as separate scalars and x + step rounds on its own.  A value
+// outside a limit, and that limit itself, both re-enter the next solve through place()'s nudge to the same point, so the
+// clamp changes no later iterate.  NaN passes through.  The clamp also hides how far an iterate left the box: the tests
+// see the iterate before the clamp through the host build (FrameStats::iterate, tests/test_stage_model_cpu.py).
+template <typename R> SK_HD R limit_clamp(R x, R lo, R hi) { return x < lo ? lo : (x > hi ? hi : x); }
+
 template <typename R> struct Vec3 { R x, y, z; };
 template <typename R> SK_HD R dot(const Vec3<R>& a, const Vec3<R>& b) {
     return Num<R>::fma_(a.z, b.z, Num<R>::fma_(a.y, b.y, a.x * b.x));
@@ -863,7 +870,10 @@ struct ChainRunner {
             ++s;
             begin_stage();
         } else {
-            const R out7[7] = {ang0, ang1, ang2, ang3, ang4, ang5, ang6};
+            const R out7[7] = {limit_clamp(ang0, io.lb(0), io.ub(0)), limit_clamp(ang1, io.lb(1), io.ub(1)),
+                               limit_clamp(ang2, io.lb(2), io.ub(2)), limit_clamp(ang3, io.lb(3), io.ub(3)),
+                               limit_clamp(ang4, io.lb(4), io.ub(4)), limit_clamp(ang5, io.lb(5), io.ub(5)),
+                               limit_clamp(ang6, io.lb(6), io.ub(6))};
             io.put_angles(t, out7, 2 * lo, hi == 3 ? 7 : 2 * hi + 2);
             ++t;
             if (t < n_frame) { begin_frame(); begin_stage(); }
@@ -885,7 +895,7 @@ template <typename R> struct ChainParams {
     R null_sq[4];    // squared norm of the inert seed slots of stages 1-4
 };
 
-struct FrameStats { int nfev[4]; int status[4]; };
+struct FrameStats { int nfev[4]; int status[4]; double iterate[7]; };   // iterate: the angles before limit_clamp
 
 // Reference (serial) composition of the four stage solves of one frame; the kernels use
 // the same pieces but interleave them across lanes.  `ang` in/out: previous frame's
@@ -912,9 +922,13 @@ SK_HD void solve_frame(const ChainParams<R>& P, const R* kp, R* ang, R* fk, Fram
             while (!S.done()) S.trip();
             if ((gn_mask & 16) && S.escape()) while (!S.done()) S.trip();
         }
-        if (s != 3) ang[ia] = S.x0;
-        ang[ib] = S.angle_b();
-        if (fs) { fs->nfev[s] = S.nfev; fs->status[s] = S.status; }
+        if (s != 3) ang[ia] = limit_clamp(S.x0, P.lb[ia], P.ub[ia]);
+        ang[ib] = limit_clamp(S.angle_b(), P.lb[ib], P.ub[ib]);
+        if (fs) {
+            fs->nfev[s] = S.nfev; fs->status[s] = S.status;
+            if (s != 3) fs->iterate[ia] = (double)S.x0;
+            fs->iterate[ib] = (double)S.angle_b();
+        }
         // next pivot = pivot + A w = target + A f
         const Vec3<R> Af = mul(A, S.res());
         piv = {(piv.x + rel.x) + Af.x, (piv.y + rel.y) + Af.y, (piv.z + rel.z) + Af.z};

@@ -222,8 +222,9 @@ __global__ void __launch_bounds__(32) leg_solve_pipe_kernel(LegArgs a, int cpw, 
                 xa = S.x0; xb = S.angle_b(); nf += (uint32_t)S.nfev;
                 worst = (S.status == ST_MAXFEV && worst > ST_MAXFEV) ? ST_MAXFEV : worst;
                 worst = (S.status == ST_NONFINITE) ? ST_NONFINITE : worst;
-                *pa_a = (s == 3) ? xb : xa;
-                *pa_b = xb;
+                const float xb_out = limit_clamp(xb, lb1, ub1);                        // (outputs inside the limits, seqik_core.cuh)
+                *pa_a = (s == 3) ? xb_out : limit_clamp(xa, lb0, ub0);
+                *pa_b = xb_out;
             }
             // joint position = pivot + A w(x) = target + A f   (q = A^T rel, f = w - q)
             const Vec3<float> Af = mul(A, S.res());
@@ -365,8 +366,8 @@ __global__ void __launch_bounds__(BLK) leg_first_frame_kernel(LegArgs a) {
         const Vec3<float> kt = map.apply({__ldg(kp + 3 * s + 3), __ldg(kp + 3 * s + 4), __ldg(kp + 3 * s + 5)}, s + 1);
         float xb; Vec3<float> w; uint32_t ne = 0u;
         serial_stage(s, k, a.gn_mask, esc, false, kt, o, A, piv, x0, x1, sa, ca, sb, cb, xb, w, ne, worst);
-        if (s < 3) ang[k.ia] = x0;
-        ang[k.ib] = xb;
+        if (s < 3) ang[k.ia] = limit_clamp(x0, k.lb0, k.ub0);
+        ang[k.ib] = limit_clamp(xb, k.lb1, k.ub1);
         put_fk_joint<kFk>(fk, s, o, w);
         auto rec = [&](int i) -> float& { return ang[(int64_t)(1 + i / 7) * a.ang_fs + i % 7]; };
         rec(4 * s) = sa; rec(4 * s + 1) = ca; rec(4 * s + 2) = sb; rec(4 * s + 3) = cb;
@@ -724,7 +725,10 @@ leg_solve_block_kernel(LegArgs a, int bulk_in, int bulk_out, int first_done) {
                     float xb; Vec3<float> w; uint32_t ne = 0u;
                     if (kRobust) serial_stage_call(s, k, a.gn_mask, esc, warm_ok, kt, o, A, piv, x0, x1, sa, ca, sb, cb, xb, w, ne, worst);
                     else serial_stage(s, k, a.gn_mask, esc, warm_ok, kt, o, A, piv, x0, x1, sa, ca, sb, cb, xb, w, ne, worst);
-                    if (s < 3) { oa[2 * s] = x0; oa[2 * s + 1] = xb; } else oa[6] = xb;
+                    // (outputs inside the limits, seqik_core.cuh limit_clamp: only the serial solver's iterates can sit an ulp
+                    //  outside; the pass's closed-form angles are admitted 1e-5 inside and its on-limit angles are placed)
+                    const float xb_out = limit_clamp(xb, K[KC_LB1], K[KC_UB1]);
+                    if (s < 3) { oa[2 * s] = limit_clamp(x0, K[KC_LB0], K[KC_UB0]); oa[2 * s + 1] = xb_out; } else oa[6] = xb_out;
                     sh.nfx[s] += ne;
                     put_fk_joint<kFk>(of, s, o, w);
                     // hand the final state on: the next pass starts from it

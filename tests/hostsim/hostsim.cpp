@@ -12,7 +12,7 @@ using namespace seqik;
 template <typename R>
 static void run_chain(const R* pose, int64_t n_frame, const R* seg, const R* lb, const R* ub,
                       const R* null_sq, const R* seed, R* angles, R* fk, int32_t* nfev, int32_t* status,
-                      int stage_mask, int gn_mask) {
+                      int stage_mask, int gn_mask, double* iterates = nullptr) {
     ChainParams<R> P;
     for (int i = 0; i < 4; ++i) { P.seg[i] = seg[i]; P.null_sq[i] = null_sq[i]; }
     for (int i = 0; i < 7; ++i) { P.lb[i] = lb[i]; P.ub[i] = ub[i]; }
@@ -23,6 +23,7 @@ static void run_chain(const R* pose, int64_t n_frame, const R* seg, const R* lb,
         solve_frame<R>(P, pose + t * 15, ang, fk ? fk + t * 27 : nullptr, &fs, stage_mask, gn_mask);
         for (int i = 0; i < 7; ++i) angles[t * 7 + i] = ang[i];
         if (nfev) for (int s = 0; s < 4; ++s) { nfev[t * 4 + s] = fs.nfev[s]; status[t * 4 + s] = fs.status[s]; }
+        if (iterates) for (int i = 0; i < 7; ++i) iterates[t * 7 + i] = fs.iterate[i];
     }
 }
 
@@ -60,6 +61,11 @@ void hostsim_chain_f32(const float* pose, int64_t n_frame, const float* seg, con
                        const float* null_sq, const float* seed, float* angles, float* fk, int32_t* nfev,
                        int32_t* status, int stage_mask, int gn_mask) {
     run_chain<float>(pose, n_frame, seg, lb, ub, null_sq, seed, angles, fk, nfev, status, stage_mask, gn_mask);
+}
+// the same with the final iterates of every stage before the output clamp (core limit_clamp), as doubles
+void hostsim_chain_iterates_f32(const float* pose, int64_t n_frame, const float* seg, const float* lb, const float* ub,
+                                const float* null_sq, const float* seed, float* angles, double* iterates, int gn_mask) {
+    run_chain<float>(pose, n_frame, seg, lb, ub, null_sq, seed, angles, nullptr, nullptr, nullptr, 0xF, gn_mask, iterates);
 }
 void hostsim_chain_f64(const double* pose, int64_t n_frame, const double* seg, const double* lb, const double* ub,
                        const double* null_sq, const double* seed, double* angles, double* fk, int32_t* nfev,
@@ -111,8 +117,8 @@ static void run_carried(const float* pose, int64_t n_frame, const float* prm, fl
                 if (!(esc && S[s].escape())) break;
             }
             xa[s] = S[s].x0; xb[s] = S[s].angle_b();
-            if (s != 3) angles[t * 7 + ia] = xa[s];
-            angles[t * 7 + ib] = xb[s];
+            if (s != 3) angles[t * 7 + ia] = limit_clamp(xa[s], lb0, ub0);
+            angles[t * 7 + ib] = limit_clamp(xb[s], lb1, ub1);
             nfev[t * 4 + s] = S[s].nfev;
             const Vec3<R> Af = mul(A, S[s].res());
             const Vec3<R> np_ = {(piv.x + rel.x) + Af.x, (piv.y + rel.y) + Af.y, (piv.z + rel.z) + Af.z};
@@ -278,8 +284,8 @@ static void run_block(const float* pose, int64_t n_frame, const float* prm, cons
                     const Vec3<R> kt = {kp[3 * (s + 1)], kp[3 * (s + 1) + 1], kp[3 * (s + 1) + 2]};
                     Vec3<R> w; uint32_t ne = 0u; int worst = ST_GTOL;
                     serial_stage(s, K[s], gn_mask, esc, ta > 0 || warm != nullptr, kt, o, Aj, pj, x0, x1, sa, ca, sb, cb, xb, w, ne, worst);
-                    if (s != 3) angles[ta * 7 + K[s].ia] = x0;
-                    angles[ta * 7 + K[s].ib] = xb;
+                    if (s != 3) angles[ta * 7 + K[s].ia] = limit_clamp(x0, K[s].lb0, K[s].ub0);
+                    angles[ta * 7 + K[s].ib] = limit_clamp(xb, K[s].lb1, K[s].ub1);
                     nfev[ta * 4 + s] = (int32_t)ne;
                     put_fk_joint<1>(fk + ta * 27, s, o, w);
                     T[s][j] = {sa, ca, sb, cb};

@@ -47,6 +47,22 @@ def solve_chain(pose, seg, lb, ub, null_sq, seed, dtype=np.float32, stage_mask=0
     return angles, fk, nfev, status
 
 
+def chain_iterates_f32(pose, seg, lb, ub, null_sq, seed, gn_mask=0):
+    """solve_chain (float32, all stages) -> angles (N,7) and the final iterates before the output clamp (N,7) float64."""
+    lib = load()
+    pose = np.ascontiguousarray(pose, dtype=np.float32)
+    n = pose.shape[0]
+    args = [np.ascontiguousarray(a, dtype=np.float32) for a in (seg, lb, ub, null_sq, seed)]
+    angles = np.zeros((n, 7), dtype=np.float32)
+    it = np.zeros((n, 7), dtype=np.float64)
+    P = ctypes.c_void_p
+    fn = lib.hostsim_chain_iterates_f32
+    fn.argtypes = [P, ctypes.c_int64, P, P, P, P, P, P, P, ctypes.c_int]
+    fn.restype = None
+    fn(pose.ctypes.data, n, *(a.ctypes.data for a in args), angles.ctypes.data, it.ctypes.data, gn_mask)
+    return angles, it
+
+
 def run_runner_f32(pose, seg, lb, ub, null_sq, seed, stage_mask=0xF, gn_mask=0):
     """Same chain through ChainRunner::step() (the kernels' per-lane state machine)."""
     lib = load()
