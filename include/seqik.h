@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define SEQIK_ABI_VERSION 9   /* 9: seqik_fk_backward_f32; 8: seqik_origin_rows_f32; 7: seqik_leg_affine_from_pose_f32; 6: schedule 3 (frame-parallel blocks), seqik_fk_expand_host_f32; 5: solver flag bits 6-7, phase periods in bits 21-27 */
+#define SEQIK_ABI_VERSION 10  /* 10: seqik_head_angles_backward_f32; 9: seqik_fk_backward_f32; 8: seqik_origin_rows_f32; 7: seqik_leg_affine_from_pose_f32; 6: schedule 3 (frame-parallel blocks), seqik_fk_expand_host_f32; 5: solver flag bits 6-7, phase periods in bits 21-27 */
 #define SEQIK_OK 0
 #define SEQIK_EINVAL (-1)
 #define SEQIK_ECUDA (-3)
@@ -220,6 +220,33 @@ int seqik_fk_backward_f32(const float* angles, const float* origin, int64_t orig
 int seqik_head_angles_f32(const float* r_head, const float* l_head, const float* neck, int64_t neck_stride,
                           const float* affine_r, const float* affine_l, const float* rest,
                           float* out, int64_t n_trial, int64_t n_frame, void* stream);
+
+/* Backward of seqik_head_angles_f32 (vector-Jacobian product): the gradient of a loss L with respect to the antenna key
+ * points and the neck, given grad_out = dL/dout.  New in this library: the reference has no gradients, so this replaces
+ * nothing in it.
+ *   r_head, l_head, neck, neck_stride, affine_r, affine_l: as for seqik_head_angles_f32.  The rest angles are additive
+ *   constants of the angles and do not enter the gradient (dL/drest_head_pitch = sum of dL/dhead_pitch,
+ *   dL/drest_antenna_pitch = -sum of dL/dantenna_pitch L and R).
+ *   grad_out     [n_trial][7][n_frame] in, the layout of seqik_head_angles_f32's out
+ *   grad_r_head, grad_l_head  [n_trial][n_frame][2][3] out (required): dL/d(base xyz, tip xyz)
+ *   grad_neck    NULL (skip), or [n_trial][n_frame][3] out: dL/dneck PER FRAME, also when neck_stride = 0 (the caller
+ *                sums over frames)
+ * The gradients are taken with respect to the points AS PASSED.  With affine rows, the points are first mapped as
+ * seqik_head_angles_f32 maps them (seqik_head_apply_f32's arithmetic), and the gradient of a raw point is the gradient of
+ * the aligned point times the row's scale, aff[3] for a base and aff[7] for a tip: one float32 multiplication, the last
+ * operation.  The affine rows themselves get no gradient.
+ * Degenerate frames: every angle is the signed angle between two vectors projected onto a coordinate plane.  Where such a
+ * projected vector has float32 squared length exactly 0, that vector's terms contribute 0 (torch.atan2's gradient at
+ * (0, 0)); when it is the roll's hor|x=0, the roll's propagation into the antenna angles is 0 as well.  A vector with a
+ * subnormal squared length (shorter than ~1e-19) is taken at squared length FLT_MIN.  For finite inputs no output is NaN
+ * or inf unless the gradient itself overflows float32.
+ * All arrays dense.  The forward's roll is recomputed with its arithmetic, so the de-rotated vectors are the forward's;
+ * results are deterministic (no atomics) and do not depend on the pointer alignment (8-byte aligned r_head / l_head /
+ * grad_r_head / grad_l_head move as 64-bit loads and stores, others as 32-bit ones, with bit-identical results). */
+int seqik_head_angles_backward_f32(const float* r_head, const float* l_head, const float* neck, int64_t neck_stride,
+                                   const float* affine_r, const float* affine_l, const float* grad_out,
+                                   float* grad_r_head, float* grad_l_head, float* grad_neck,
+                                   int64_t n_trial, int64_t n_frame, void* stream);
 
 /* AlignPose statistics: mean of the 0.45 and 0.55 quantiles (numpy "linear" interpolation) of each series.
  * Replaces _get_mean_quantile over the series built by AlignPose.get_fixed_pos / get_mean_length

@@ -2,7 +2,7 @@
 
 Algorithmic bytes per unit (DESIGN.md 5.3): fk 28+12+108 B/leg-frame (origin per frame), fk backward 28+108 in and 28+12
 (+16 with the lengths) out, head 48+28 B/frame (+12 with a
-per-frame neck), align_apply 60+60 B/leg-frame, leg_series 60 in + 28 out, mid_quantile 4 B/element read (4 ranks x
+per-frame neck), head backward 48+28 in and 48+12 out, align_apply 60+60 B/leg-frame, leg_series 60 in + 28 out, mid_quantile 4 B/element read (4 ranks x
 4 radix passes re-read the series: from L2 when it fits)."""
 import json, sys
 from pathlib import Path
@@ -79,6 +79,22 @@ nf = n_trial * n_frame * 6
 r = torch.randn((n_trial, 6 * n_frame, 2, 3), device="cuda", generator=g); l = torch.randn((n_trial, 6 * n_frame, 2, 3), device="cuda", generator=g)
 neck = torch.randn((n_trial, 3), device="cuda", generator=g); rest = torch.zeros((n_trial, 2), device="cuda")
 report("head_kernel", timeit(lambda: engine.head_angles(r, l, neck, rest)), nf * (48 + 28), nf, "frames")
+# head-angle backward: r_head, l_head + grad_out in, grad_r_head, grad_l_head + grad_neck (per frame) out
+g_head = torch.randn((n_trial, 7, 6 * n_frame), device="cuda", generator=g)
+report("head_backward_kernel", timeit(lambda: engine.head_angles_backward(r, l, neck, g_head)), nf * (48 + 28 + 48 + 12), nf, "frames")
+# forward + VJP (r_head, l_head): through engine.head_angles' autograd, and through torch autograd of the same angles in
+# float64 torch ops (tests/model_head_torch.py).  Bytes: those of the two kernels.
+r_req, l_req = r.clone().requires_grad_(), l.clone().requires_grad_()
+report("head_angles + backward through autograd (kernels)",
+       timeit(lambda: torch.autograd.grad(engine.head_angles(r_req, l_req, neck, rest), [r_req, l_req], g_head)),
+       nf * (48 + 28 + 48 + 28 + 48), nf, "frames")
+import model_head_torch
+r64, l64, n64 = r.double().requires_grad_(), l.double().requires_grad_(), neck.double()[:, None]
+g64 = g_head.double().permute(1, 0, 2)
+report("float64 torch-ops head angles + torch autograd VJP (reference point)",
+       timeit(lambda: torch.autograd.grad(model_head_torch.head_angles_torch(r64, l64, n64, 0.0, 0.0), [r64, l64], g64), reps=3),
+       nf * (48 + 28 + 48 + 28 + 48), nf, "frames")
+del g_head, r_req, l_req, r64, l64, n64, g64
 th = torch.randn((n_trial, 6 * n_frame, 3, 3), device="cuda", generator=g); hc = torch.rand((n_trial, 5), device="cuda", generator=g) + 0.5
 report("head_affine (series fp64 + radix select + affine)", timeit(lambda: engine.head_affine(r, th, hc)), nf * (24 + 36 + 20 + 20), nf, "frames")
 report("head_apply_kernel", timeit(lambda: engine.head_apply(r, torch.rand((n_trial, 8), device="cuda") + 0.5)), nf * 48, nf, "frames")

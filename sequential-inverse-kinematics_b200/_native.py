@@ -12,7 +12,7 @@ import numpy as np
 _HERE = Path(__file__).resolve().parent
 LIB_PATH = _HERE / "csrc" / "libseqik_sm100.so"
 
-ABI_VERSION = 9
+ABI_VERSION = 10
 CHAIN_PARAM_FLOATS = 32
 FLAG_ESCAPE = 1 << 4
 FLAG_SKIP_CONFIRM = 1 << 5
@@ -45,6 +45,7 @@ _SIGNATURES = {
     "seqik_fk_f32": (_int, [_vp, _vp, _i64, _vp, _vp, _i64, _i64, _vp]),
     "seqik_fk_backward_f32": (_int, [_vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _vp]),
     "seqik_head_angles_f32": (_int, [_vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp, _i64, _i64, _vp]),
+    "seqik_head_angles_backward_f32": (_int, [_vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _vp]),
     "seqik_mid_quantile_f32": (_int, [_vp, _vp, _vp, _vp, _i64, _i64, _vp]),
     "seqik_leg_series_f32": (_int, [_vp, _i64, _i64, _vp, _i64, _i64, _vp]),
     "seqik_leg_affine_f32": (_int, [_vp, _vp, _int, _vp, _i64, _vp]),

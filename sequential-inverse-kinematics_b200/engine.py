@@ -258,11 +258,8 @@ def _fk_function():
     return _FK_FUNCTION
 
 
-def head_angles(r_head, l_head, neck, rest, affine_r=None, affine_l=None):
-    """r_head, l_head (n_trial, n_frame, 2, 3); neck (n_trial, n_frame, 3) or (n_trial, 3); rest (n_trial, 2)
-    -> (n_trial, 7, n_frame): head roll, pitch, yaw, antenna yaw L, pitch L, yaw R, pitch R."""
-    torch = N.require_cuda()
-    lib = N.load_library()
+def _head_inputs(r_head, l_head, neck, affine_r, affine_l):
+    """Checks of the head-angle inputs -> (n_trial, n_frame, neck stride)."""
     r_head = _check(r_head, "r_head", (2, 3))
     l_head = _check(l_head, "l_head", (2, 3))
     if r_head.dim() != 4 or r_head.shape != l_head.shape:
@@ -275,16 +272,101 @@ def head_angles(r_head, l_head, neck, rest, affine_r=None, affine_l=None):
         stride = 0
     else:
         raise ValueError("neck must be (n_trial, n_frame, 3) or (n_trial, 3)")
-    rest = _check(rest, "rest", (2,))
     if affine_r is not None:
         _check(affine_r, "affine_r", (8,))
         _check(affine_l, "affine_l", (8,))
+    return n_trial, n_frame, stride
+
+
+def head_angles(r_head, l_head, neck, rest, affine_r=None, affine_l=None):
+    """r_head, l_head (n_trial, n_frame, 2, 3); neck (n_trial, n_frame, 3) or (n_trial, 3); rest (n_trial, 2)
+    -> (n_trial, 7, n_frame): head roll, pitch, yaw, antenna yaw L, pitch L, yaw R, pitch R.
+
+    Differentiable: when grad mode is on and ``r_head``, ``l_head``, ``neck`` or ``rest`` requires grad, the result
+    carries a ``grad_fn`` whose backward is the ``seqik_head_angles_backward_f32`` kernel (see ``head_angles_backward``).
+    An (n_trial, 3) neck gets the sum over frames; ``rest`` gets dL/drest[:, 0] = the sum of dL/dhead_pitch and
+    dL/drest[:, 1] = minus the sums of dL/dantenna_pitch L and R.  The affine rows are constants of the backward: one
+    that requires grad raises ValueError.  First derivatives only: a second backward raises.  Without inputs that
+    require grad the call is the plain kernel launch."""
+    torch = N.require_cuda()
+    if torch.is_grad_enabled():
+        if any(isinstance(t, torch.Tensor) and t.requires_grad for t in (affine_r, affine_l)):
+            raise ValueError("head_angles: the affine rows have no gradient; pass them detached")
+        if any(isinstance(t, torch.Tensor) and t.requires_grad for t in (r_head, l_head, neck, rest)):
+            return _head_function().apply(r_head, l_head, neck, rest, affine_r, affine_l)
+    return _head_angles(torch, r_head, l_head, neck, rest, affine_r, affine_l)
+
+
+def _head_angles(torch, r_head, l_head, neck, rest, affine_r, affine_l):
+    lib = N.load_library()
+    n_trial, n_frame, stride = _head_inputs(r_head, l_head, neck, affine_r, affine_l)
+    rest = _check(rest, "rest", (2,))
     out = torch.empty((n_trial, 7, n_frame), dtype=torch.float32, device=r_head.device)
     with torch.cuda.device(r_head.device):
         rc = lib.seqik_head_angles_f32(N.ptr(r_head), N.ptr(l_head), N.ptr(neck), stride, N.ptr(affine_r), N.ptr(affine_l),
                                        N.ptr(rest), N.ptr(out), n_trial, n_frame, N.stream_ptr(torch, r_head.device))
     N.check(rc, "seqik_head_angles_f32")
     return out
+
+
+def head_angles_backward(r_head, l_head, neck, grad_out, affine_r=None, affine_l=None, want_neck: bool = True):
+    """Vector-Jacobian product of ``head_angles``: grad_out (n_trial, 7, n_frame) = dL/dangles ->
+    (grad_r_head (n_trial, n_frame, 2, 3), grad_l_head (n_trial, n_frame, 2, 3), grad_neck (n_trial, n_frame, 3) | None).
+    grad_neck is per frame also for an (n_trial, 3) neck: sum over frames there.  The gradients are those of the points
+    as passed: with affine rows, the aligned points' gradients times the rows' scales (include/seqik.h).  The rest angles
+    are additive constants and the affine rows get no gradient."""
+    torch = N.require_cuda()
+    lib = N.load_library()
+    n_trial, n_frame, stride = _head_inputs(r_head, l_head, neck, affine_r, affine_l)
+    grad_out = _check(grad_out, "grad_out", (n_frame,))
+    if tuple(grad_out.shape) != (n_trial, 7, n_frame):
+        raise ValueError(f"grad_out must be ({n_trial}, 7, {n_frame}), got {tuple(grad_out.shape)}")
+    dev = r_head.device
+    grad_r = torch.empty((n_trial, n_frame, 2, 3), dtype=torch.float32, device=dev)
+    grad_l = torch.empty((n_trial, n_frame, 2, 3), dtype=torch.float32, device=dev)
+    grad_neck = torch.empty((n_trial, n_frame, 3), dtype=torch.float32, device=dev) if want_neck else None
+    with torch.cuda.device(dev):
+        rc = lib.seqik_head_angles_backward_f32(N.ptr(r_head), N.ptr(l_head), N.ptr(neck), stride, N.ptr(affine_r),
+                                                N.ptr(affine_l), N.ptr(grad_out), N.ptr(grad_r), N.ptr(grad_l),
+                                                N.ptr(grad_neck), n_trial, n_frame, N.stream_ptr(torch, dev))
+    N.check(rc, "seqik_head_angles_backward_f32")
+    return grad_r, grad_l, grad_neck
+
+
+_HEAD_FUNCTION = None
+
+
+def _head_function():
+    """The torch.autograd.Function of head_angles (built on first use: torch is imported lazily)."""
+    global _HEAD_FUNCTION
+    if _HEAD_FUNCTION is not None:
+        return _HEAD_FUNCTION
+    import torch
+    from torch.autograd.function import once_differentiable
+
+    class HeadAngles(torch.autograd.Function):
+        @staticmethod
+        def forward(ctx, r_head, l_head, neck, rest, affine_r, affine_l):
+            ctx.save_for_backward(r_head, l_head, neck, affine_r, affine_l)
+            return _head_angles(torch, r_head, l_head, neck, rest, affine_r, affine_l)
+
+        @staticmethod
+        @once_differentiable
+        def backward(ctx, grad_out):
+            r_head, l_head, neck, affine_r, affine_l = ctx.saved_tensors
+            need_r, need_l, need_neck, need_rest = ctx.needs_input_grad[:4]
+            grad_out = grad_out.contiguous()
+            gr = gl = gn = g_rest = None
+            if need_r or need_l or need_neck:
+                gr, gl, gn = head_angles_backward(r_head, l_head, neck, grad_out, affine_r, affine_l, want_neck=need_neck)
+                if need_neck and neck.dim() == 2:
+                    gn = gn.sum(dim=1)
+            if need_rest:
+                g_rest = torch.stack([grad_out[:, 1].sum(-1), -(grad_out[:, 4] + grad_out[:, 6]).sum(-1)], dim=1)
+            return (gr if need_r else None), (gl if need_l else None), gn, g_rest, None, None
+
+    _HEAD_FUNCTION = HeadAngles
+    return _HEAD_FUNCTION
 
 
 def mid_quantile(series, counts=None):
