@@ -158,10 +158,18 @@ int seqik_leg_solve_f32(const float* pose, int64_t pose_chain_stride, int64_t po
  *           sums over the joints by butterfly shuffles; up to 4 chains per warp).  Same iteration, different summation
  *           order; other bits must be 0
  *
+ *   status  per chain: -1 if some frame was skipped (a non-finite key point; it takes precedence over everything else),
+ *           else 0 if some solve stopped at the evaluation limit (100 * 9), else 1.  A skipped frame counts one evaluation
+ *           in nfev, its angles are the ones it was seeded with (the previous frame's, or the seed for frame 0), its fk
+ *           rows are those angles placed at its own origin (so not finite when the origin is not), and the next frame
+ *           starts from the same angles: the frames after it are bit-identical to a call without the skipped frame.
+ *           Returned angles lie strictly inside the limits in the working precision.
+ *
  * The reference's generic solve is under-determined (3 equations, 7 unknowns) and its answer depends on rounding noise
  * (DESIGN.md 5.4): this entry point restates the same iteration, reproduces the reference solve by solve from the same
  * seed (tests) and reaches the same claw residual, but a free-running recording follows its own path on the
- * self-motion manifold. */
+ * self-motion manifold.  In FP64 both mappings take the same iterates as the host build of seqik_generic.cuh on every
+ * solve that rounding-level perturbations do not change (tests/test_gpu_generic_cert.py). */
 int seqik_leg_solve_generic_f32(const float* pose, int64_t pose_chain_stride, int64_t pose_frame_stride, int32_t target_row,
                                 const float* params,
                                 float* angles, int64_t ang_chain_stride, int64_t ang_frame_stride,

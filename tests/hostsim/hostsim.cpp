@@ -332,6 +332,27 @@ static void run_generic(const R* pose, int64_t n_frame, const R* prm, const R* t
     }
 }
 
+// n independent single solves, each with its own constants row prm (n,32) (seed from 18..24), target (n,3) as the kernel
+// forms it (key point minus origin, already rounded) -> angles (n,7), fk rows relative to the origin (n,9,3), nfev, status
+template <typename R>
+static void run_generic_solves(int64_t n, const R* prm, const R* target, R* angles, R* fk, int32_t* nfev, int32_t* status) {
+    for (int64_t k = 0; k < n; ++k) {
+        const R* pk = prm + k * 32;
+        GenericSolve<R> S;
+        for (int i = 0; i < 7; ++i) S.x[i] = pk[18 + i];
+        S.start(pk, Vec3<R>{target[3 * k], target[3 * k + 1], target[3 * k + 2]}, pk[25]);
+        while (!S.done()) S.trip();
+        for (int i = 0; i < 7; ++i) angles[k * 7 + i] = S.x[i];
+        nfev[k] = S.nfev; status[k] = S.status;
+        Vec3<R> org[3], claw;
+        S.joints(org, &claw);
+        R* o = fk + k * 27;
+        for (int r = 0; r < 12; ++r) o[r] = R(0);
+        const Vec3<R> rows[5] = {org[0], org[0], org[1], org[2], claw};
+        for (int r = 0; r < 5; ++r) { o[12 + 3 * r] = rows[r].x; o[13 + 3 * r] = rows[r].y; o[14 + 3 * r] = rows[r].z; }
+    }
+}
+
 extern "C" {
 void hostsim_generic_f32(const float* pose, int64_t n_frame, const float* prm, const float* teacher, float* angles,
                          float* fk, int32_t* nfev, int32_t* status) {
@@ -340,6 +361,14 @@ void hostsim_generic_f32(const float* pose, int64_t n_frame, const float* prm, c
 void hostsim_generic_f64(const double* pose, int64_t n_frame, const double* prm, const double* teacher, double* angles,
                          double* fk, int32_t* nfev, int32_t* status) {
     run_generic<double>(pose, n_frame, prm, teacher, angles, fk, nfev, status);
+}
+void hostsim_generic_solves_f32(int64_t n, const float* prm, const float* target, float* angles, float* fk, int32_t* nfev,
+                                int32_t* status) {
+    run_generic_solves<float>(n, prm, target, angles, fk, nfev, status);
+}
+void hostsim_generic_solves_f64(int64_t n, const double* prm, const double* target, double* angles, double* fk,
+                                int32_t* nfev, int32_t* status) {
+    run_generic_solves<double>(n, prm, target, angles, fk, nfev, status);
 }
 }
 

@@ -142,3 +142,24 @@ def solve_generic(pose2, prm, teacher=None, dtype=np.float32, want_fk=True):
     fn(pose2.ctypes.data, n, prm.ctypes.data, None if teacher is None else teacher.ctypes.data, angles.ctypes.data,
        fk.ctypes.data if want_fk else None, nfev.ctypes.data, status.ctypes.data)
     return angles, fk, nfev, status
+
+
+def solve_generic_many(prm, target, dtype=np.float64):
+    """n independent generic solves on the host build: prm (n,32) constants rows (seed in 18..24, null_sq in 25), target
+    (n,3) claw minus origin as the kernel forms it -> angles (n,7), fk rows relative to the origin (n,9,3), nfev (n,),
+    status (n,)."""
+    lib = load()
+    fn = lib.hostsim_generic_solves_f32 if dtype == np.float32 else lib.hostsim_generic_solves_f64
+    prm = np.ascontiguousarray(prm, dtype=dtype).reshape(-1, 32)
+    target = np.ascontiguousarray(target, dtype=dtype).reshape(-1, 3)
+    n = prm.shape[0]
+    assert target.shape[0] == n
+    angles = np.zeros((n, 7), dtype=dtype)
+    fk = np.zeros((n, 9, 3), dtype=dtype)
+    nfev = np.zeros(n, dtype=np.int32)
+    status = np.zeros(n, dtype=np.int32)
+    P = ctypes.c_void_p
+    fn.argtypes = [ctypes.c_int64, P, P, P, P, P, P]
+    fn.restype = None
+    fn(n, prm.ctypes.data, target.ctypes.data, angles.ctypes.data, fk.ctypes.data, nfev.ctypes.data, status.ctypes.data)
+    return angles, fk, nfev, status
