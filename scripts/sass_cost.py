@@ -12,7 +12,7 @@ from collections import defaultdict
 from pathlib import Path
 
 
-def disasm(path, kernel):
+def disasm(path, kernel, flags=("-g", "-hex")):
     path = Path(path)
     tmp = Path(tempfile.mkdtemp())
     if path.suffix != ".cubin":
@@ -21,7 +21,7 @@ def disasm(path, kernel):
     else:
         cubins = [path]
     for cb in cubins:
-        txt = subprocess.run(["nvdisasm", "-g", "-hex", str(cb)], capture_output=True, text=True).stdout
+        txt = subprocess.run(["nvdisasm", *flags, str(cb)], capture_output=True, text=True).stdout
         m = re.search(r"^\.text\.(\S*%s\S*):" % re.escape(kernel), txt, re.M)
         if m:
             start = m.start()

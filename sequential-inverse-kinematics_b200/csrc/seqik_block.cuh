@@ -110,6 +110,19 @@ template <typename R> SK_HD int warm_guess(R n_sa, R n_ca, R sl0, R cl0, R su0, 
     return (below == above) ? WC_INTERIOR : below ? WC_LO : WC_HI;
 }
 
+// ---- piece 4a: the interior half of warm_case() below: WC_INTERIOR when the serial solver ends at the interior candidate,
+// else WC_NONE; x0 / x1 = the candidate's angles either way.  For a candidate guessed interior this is the whole decision:
+// warm_case() returns a limit only when it matches the guess.
+template <typename R>
+SK_HD int warm_case_interior(bool enable, R xp0, R xp1, const WarmMove<R>& mv, bool cond, R lb0, R ub0, R lb1s, R ub1s,
+                             R& x0, R& x1) {
+    const R m = R(1e-5);
+    const R nx0 = xp0 + mv.dA, nx1 = xp1 + mv.dB;
+    const bool in_a = (nx0 - lb0 > m) & (ub0 - nx0 > m), in_b = (nx1 - lb1s > m) & (ub1s - nx1 > m);
+    x0 = nx0; x1 = nx1;
+    return (enable & mv.small_a & mv.small_b & cond & in_a & in_b) ? WC_INTERIOR : WC_NONE;
+}
+
 // ---- piece 4: the decision warm_step() takes, given the exact placed warm-start angles (xp0, xp1).  `guess`: the case the
 // candidate data (dB2, small_b2, lim_ok_q) was prepared for.  Returns WC_INTERIOR / WC_LO / WC_HI when the serial solver ends
 // at that candidate, WC_NONE when it would not (or when it would take a limit the data was not prepared for): the caller
@@ -119,11 +132,8 @@ SK_HD int warm_case(bool enable, bool have_bt, bool one_var, R xp0, R xp1, const
                     R lb0, R ub0, R lb1s, R ub1s, int guess, R dB2, bool small_b2, bool lim_ok_q, R& x0, R& x1) {
     typedef Num<R> N;
     const R m = R(1e-5);
-    const R nx0 = xp0 + mv.dA, nx1 = xp1 + mv.dB;
-    const bool in_a = (nx0 - lb0 > m) & (ub0 - nx0 > m), in_b = (nx1 - lb1s > m) & (ub1s - nx1 > m);
-    const bool ok = enable & mv.small_a & mv.small_b & cond & in_a & in_b;
-    x0 = nx0; x1 = nx1;
-    if (ok) return WC_INTERIOR;
+    if (warm_case_interior(enable, xp0, xp1, mv, cond, lb0, ub0, lb1s, ub1s, x0, x1) == WC_INTERIOR) return WC_INTERIOR;
+    const R nx0 = x0;
     const bool below = nx0 - lb0 <= m, above = ub0 - nx0 <= m;
     if (!(enable & have_bt & !one_var & (below != above) & mv.small_a)) return WC_NONE;
     const bool lo = below;

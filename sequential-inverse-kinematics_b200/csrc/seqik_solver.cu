@@ -510,7 +510,8 @@ leg_solve_block_kernel(LegArgs a, int bulk_in, int bulk_out, int first_done) {
             const bool act = lane >= j0 && lane < nv;
             // results of the pass per lane and stage
             float Tsa[4], Tca[4], Tsb[4], Tcb[4];                  // final sin/cos per stage (speculated)
-            float dA[4], dB[4], dB2[4]; uint32_t bits = 0u;        // per stage: bit 0 small_a, 1 small_a & small_b & cond, 2 small_b2 & lim ok_q, 5-6 guess
+            float dA[4], dB[4]; uint32_t bits = 0u;                // per stage (byte s): bit 0 small_a & small_b & (cond or lim ok_q), 5-6 guess
+            uint32_t lim_stages = 0u;                              // bit s: some active lane guessed a limit in stage s (warp-uniform)
             Vec3<float> npv[4];                                    // end point of each stage relative to the origin
             // ================= pass =================
             {
@@ -544,13 +545,14 @@ leg_solve_block_kernel(LegArgs a, int bulk_in, int bulk_out, int first_done) {
                     if (!one_var) g = warm_guess(cd.n_sa, cd.n_ca, K[KC_SL0], K[KC_CL0], K[KC_SU0], K[KC_CU0]);
                     float tsa = cd.n_sa, tca = cd.n_ca, tsb = cd.n_sb, tcb = cd.n_cb;
                     Vec3<float> f = cd.f;
-                    bool limq = false;
+                    bool cq = cd.cond;                             // the admission tests of this lane's candidate that depend on the target alone
                     const bool any_lim = !one_var && __any_sync(full, act && g != WC_INTERIOR);
+                    if (any_lim) lim_stages |= 1u << s;
                     if (any_lim && g != WC_INTERIOR) {             // (warp-uniform outer test: the block is skipped when no lane needs it)
                         const bool lo = g == WC_LO;
                         tsa = lo ? K[KC_SL0] : K[KC_SU0]; tca = lo ? K[KC_CL0] : K[KC_CU0];
                         const WarmLimit<float> lc = warm_limit(q, L, lo, tsa, tca, sgn);
-                        tsb = lc.c_sb; tcb = lc.c_cb; f = lc.f; limq = lc.ok_q;
+                        tsb = lc.c_sb; tcb = lc.c_cb; f = lc.f; cq = lc.ok_q;
                     }
                     if (kRobust && one_var) {
                         // The one-variable stage sitting ON a limit (TiTa_pitch = 0 for long stretches of a real recording): while
@@ -584,20 +586,22 @@ leg_solve_block_kernel(LegArgs a, int bulk_in, int bulk_out, int first_done) {
                     if (!fold_a) { psa = __shfl_up_sync(full, tsa, 1); pca = __shfl_up_sync(full, tca, 1); }
                     float psb = __shfl_up_sync(full, tsb, 1), pcb = __shfl_up_sync(full, tcb, 1);
                     if (lane == j0) { psa = Psa; pca = Pca; psb = Psb; pcb = Pcb; }
-                    const WarmMove<float> mv = warm_move(cd.n_sa, cd.n_ca, cd.n_sb, cd.n_cb, psa, pca, psb, pcb);
-                    float d2 = 0.f; bool sm2 = false;
-                    if (any_lim && g != WC_INTERIOR) warm_limit_move(tsb, tcb, psb, pcb, d2, sm2);
-                    dA[s] = mv.dA; dB[s] = mv.dB; dB2[s] = d2;
-                    // (what the verification needs of the tests that depend on the target alone: small_a on its own, the
-                    //  conjunction small_a & small_b & cond of the interior case, the conjunction small_b2 & ok_q of the limit case)
-                    bits = (bits & ~(0xffu << (8 * s)))
-                           | (((mv.small_a ? 1u : 0u) | ((mv.small_a & mv.small_b & cd.cond) ? 2u : 0u) | ((sm2 & limq) ? 4u : 0u)
-                               | ((uint32_t)g << 5)) << (8 * s));
+                    // The first angle's move is the interior candidate's in every case (warm_case tests it against the limits).
+                    // The second angle's move is that of the lane's own candidate, (tsb, tcb): for an interior guess warm_step's
+                    // interior move, for a limit guess its on-limit move (warm_limit_move is the same arithmetic) -- a lane
+                    // uses only the one of its guess, in the series and in the verification alike.
+                    const WarmMove<float> mv = warm_move(cd.n_sa, cd.n_ca, tsb, tcb, psa, pca, psb, pcb);
+                    dA[s] = mv.dA; dB[s] = mv.dB;
+                    // (what the verification needs of the tests that depend on the target alone: the half of warm_case that can
+                    //  confirm the guess uses them only in the conjunction small_a & small_b & cq of the guessed candidate.  The
+                    //  other half cannot confirm it whatever this bit says: a limit guess fails the interior half when the first
+                    //  angle is inside its box (WC_INTERIOR or WC_NONE), and that half is false when it is not; an interior
+                    //  guess never matches the limit half.)
+                    bits |= (((mv.small_a & mv.small_b & cq) ? 1u : 0u) | ((uint32_t)g << 5)) << (8 * s);
                     if (act) {
                         float2 va = make_float2(mv.dA, 1.f), vb = make_float2(mv.dB, 1.f);
-                        if (any_lim && (g == WC_LO || g == WC_HI)) {         // (rare: behind the warp-uniform test)
-                            va = make_float2(g == WC_LO ? K[KC_LB0P] : K[KC_UB0P], 0.f); vb.x = d2;
-                        }
+                        if (any_lim && (g == WC_LO || g == WC_HI))           // (rare: behind the warp-uniform test)
+                            va = make_float2(g == WC_LO ? K[KC_LB0P] : K[KC_UB0P], 0.f);
                         if (kRobust && g == WC_STAYS) vb.x = 0.f;
                         if (!one_var) sh.acc_vk[s][lane] = va;
                         sh.acc_vk[3 + s][lane] = vb;
@@ -640,9 +644,10 @@ leg_solve_block_kernel(LegArgs a, int bulk_in, int bulk_out, int first_done) {
             if (kRobust && s_start > 0) {                                     // (rare) the stages that stood: their verification data
 #pragma unroll
                 for (int s = 0; s < 3; ++s)
-                    if (s < s_start) { dA[s] = stash_f[9 * s + 4]; dB[s] = stash_f[9 * s + 5]; dB2[s] = stash_f[9 * s + 6]; }
+                    if (s < s_start) { dA[s] = stash_f[9 * s + 4]; dB[s] = stash_f[9 * s + 5]; }
                 const uint32_t keep = 0xffffffffu << (8 * s_start);          // bytes of the stages this pass recomputed
                 bits = (bits & keep) | (__float_as_uint(stash_a[3]) & ~keep);
+                lim_stages |= (1u << s_start) - 1u;                           // (the whole decision for the stages that stood)
             }
             float ox0[4], ox1[4];
             int fs = 4;                                                       // first stage of this lane whose speculation does not hold
@@ -652,12 +657,16 @@ leg_solve_block_kernel(LegArgs a, int bulk_in, int bulk_out, int first_done) {
                 const uint32_t bs = bits >> (8 * s);
                 const int g = (int)((bs >> 5) & 3u);
                 const float xp0 = (s < 3) ? sh.acc_x[s < 3 ? s : 0][lane + 1] : 0.f, xp1 = sh.acc_x[3 + s][lane + 1];
-                WarmMove<float> mv; mv.dA = (s < 3 || kRobust) ? dA[s] : 0.f; mv.dB = dB[s]; mv.small_a = bs & 1u; mv.small_b = bs & 2u;
-                int wc = warm_case(enable_t, s < 3 && K[KC_HAVE_BT] != 0.f, s == 3, xp0, xp1, mv,
-                                   true, (s < 3 || kRobust) ? K[KC_LB0] : -inf, (s < 3 || kRobust) ? K[KC_UB0] : inf, K[KC_LB1S], K[KC_UB1S], g, dB2[s],
-                                   (bs & 4u) != 0u, true, ox0[s], ox1[s]);
-                if (s == 3 && g == WC_STAYS) { wc = WC_STAYS; ox0[s] = 0.f; ox1[s] = xp1; }      // decided exactly in the pass
-                fs = (wc != g) ? s : fs;
+                WarmMove<float> mv; mv.dA = (s < 3 || kRobust) ? dA[s] : 0.f; mv.dB = dB[s]; mv.small_a = bs & 1u; mv.small_b = true;
+                const float lb0 = (s < 3 || kRobust) ? K[KC_LB0] : -inf, ub0 = (s < 3 || kRobust) ? K[KC_UB0] : inf;
+                bool held;                                                    // the decision warm_step takes is the guessed one
+                if (lim_stages & (1u << s))                                   // (warp-uniform) some lane guessed a limit: the whole decision
+                    held = warm_case(enable_t, s < 3 && K[KC_HAVE_BT] != 0.f, s == 3, xp0, xp1, mv, true, lb0, ub0, K[KC_LB1S], K[KC_UB1S],
+                                     g, dB[s], true, true, ox0[s], ox1[s]) == g;
+                else                                                          // every active lane guessed interior: its half decides
+                    held = warm_case_interior(enable_t, xp0, xp1, mv, true, lb0, ub0, K[KC_LB1S], K[KC_UB1S], ox0[s], ox1[s]) == WC_INTERIOR;
+                if (kRobust && s == 3 && g == WC_STAYS) { held = true; ox0[s] = 0.f; ox1[s] = xp1; }      // decided exactly in the pass
+                fs = held ? fs : s;
             }
             const unsigned failed = __ballot_sync(full, act && fs < 4);
             const int j = failed ? __ffs((int)failed) - 1 : nv;              // first lane whose speculation does not hold
@@ -689,7 +698,7 @@ leg_solve_block_kernel(LegArgs a, int bulk_in, int bulk_out, int first_done) {
 #pragma unroll
                 for (int s = 0; s < 3; ++s) {
                     stash_f[9 * s] = Tsa[s]; stash_f[9 * s + 1] = Tca[s]; stash_f[9 * s + 2] = Tsb[s]; stash_f[9 * s + 3] = Tcb[s];
-                    stash_f[9 * s + 4] = dA[s]; stash_f[9 * s + 5] = dB[s]; stash_f[9 * s + 6] = dB2[s];
+                    stash_f[9 * s + 4] = dA[s]; stash_f[9 * s + 5] = dB[s];
                     stash_f[9 * s + 7] = npv[s].x; stash_f[9 * s + 8] = npv[s].y; stash_a[s] = npv[s].z;
                 }
                 stash_a[3] = __uint_as_float(bits);
