@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define SEQIK_ABI_VERSION 10  /* 10: seqik_head_angles_backward_f32; 9: seqik_fk_backward_f32; 8: seqik_origin_rows_f32; 7: seqik_leg_affine_from_pose_f32; 6: schedule 3 (frame-parallel blocks), seqik_fk_expand_host_f32; 5: solver flag bits 6-7, phase periods in bits 21-27 */
+#define SEQIK_ABI_VERSION 11  /* 11: seqik_pchip_resample_backward_f32/_f64; 10: seqik_head_angles_backward_f32; 9: seqik_fk_backward_f32; 8: seqik_origin_rows_f32; 7: seqik_leg_affine_from_pose_f32; 6: schedule 3 (frame-parallel blocks), seqik_fk_expand_host_f32; 5: solver flag bits 6-7, phase periods in bits 21-27 */
 #define SEQIK_OK 0
 #define SEQIK_EINVAL (-1)
 #define SEQIK_ECUDA (-3)
@@ -331,6 +331,30 @@ int seqik_pchip_resample_f32(const float* in, float* out, int64_t n_block, int64
                              double original_ts, double new_ts, void* stream);
 int seqik_pchip_resample_f64(const double* in, double* out, int64_t n_block, int64_t n, int64_t m, int64_t width,
                              double original_ts, double new_ts, void* stream);
+
+/* Backward of seqik_pchip_resample_f32/_f64 (vector-Jacobian product): grad_in = dL/din given grad_out = dL/dout.  New in
+ * this library: the reference has no gradients, so this replaces nothing in it.
+ *   in [n_block][n][width], grad_out [n_block][m][width] in, grad_in [n_block][n][width] out; sizes, limits and error
+ *   codes are those of the forward (n >= 2, positive steps, width <= 256; n_block = 0 or width = 0 returns OK).
+ *   grad_in is written in full, zeros included (it may be uninitialised).  in must hold the values the forward was
+ *   given (finite; the host wrapper zeroes +-inf as for the forward and gives the replaced samples gradient 0).
+ * The VJP is taken at the samples the forward evaluated: the same sample-to-interval assignment (the float64 interval
+ * search) and the same offsets s from the left knot (float64; in float32 the forward's fmaf(u - u_lo, (float)new_ts, s0)).
+ * A sample in interval k is y_k + d_k s + c1 s^2 + c0 s^3 with h = original_ts, m_k = (y_{k+1} - y_k) / h,
+ * c1 = (3 m_k - 2 d_k - d_{k+1}) / h and c0 = (d_k + d_{k+1} - 2 m_k) / h^2.  The knot slopes d are differentiated on the
+ * branch the forward took, its decisions recomputed with its arithmetic (in float32 with its __fdividef): an interior
+ * d = 2ab / (a + b) of the neighbouring secants, or 0 (gradient 0) where they differ in sign or one is 0; an end slope
+ * (3 m0 - m1) / 2 (partials 3/2 and -1/2), or zeroed (gradient 0), or clamped to 3 m0 (d/dm0 = 3, d/dm1 = 0); for n = 2
+ * d_0 = d_1 = m_0.
+ * Float summation order: per interval the moments M_p = sum g s^p (p = 0..3) in ascending sample order; then per knot
+ * dL/dd_i = (right term of interval i-1) + (left term of interval i), times the slope partials; per interval
+ * dL/dm_k = direct term + (knot k) + (knot k+1) [+ (knot 0) for k = 1] [+ (knot n-1) for k = n-3]; and
+ * dL/dy_i = M0[i] + (dL/dm_{i-1} - dL/dm_i) * (1 / h).  Deterministic (no atomics); the result does not depend on the
+ * width's launch path, the pointers' alignment, or whether grad_out is staged in shared memory or read directly. */
+int seqik_pchip_resample_backward_f32(const float* in, const float* grad_out, float* grad_in, int64_t n_block, int64_t n,
+                                      int64_t m, int64_t width, double original_ts, double new_ts, void* stream);
+int seqik_pchip_resample_backward_f64(const double* in, const double* grad_out, double* grad_in, int64_t n_block,
+                                      int64_t n, int64_t m, int64_t width, double original_ts, double new_ts, void* stream);
 
 /* Strided copy between host (pinned) and device buffers: `height` rows of `width_bytes`, row pitches in bytes.
  * direction 1 = host to device, 2 = device to host.  Plumbing for the chunked host pipeline (a frame range of a

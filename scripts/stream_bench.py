@@ -2,7 +2,8 @@
 
 Algorithmic bytes per unit (DESIGN.md 5.3): fk 28+12+108 B/leg-frame (origin per frame), fk backward 28+108 in and 28+12
 (+16 with the lengths) out, head 48+28 B/frame (+12 with a
-per-frame neck), head backward 48+28 in and 48+12 out, align_apply 60+60 B/leg-frame, leg_series 60 in + 28 out, mid_quantile 4 B/element read (4 ranks x
+per-frame neck), head backward 48+28 in and 48+12 out, pchip n+m values per block row and channel, pchip backward n+m in
+and n out, align_apply 60+60 B/leg-frame, leg_series 60 in + 28 out, mid_quantile 4 B/element read (4 ranks x
 4 radix passes re-read the series: from L2 when it fits)."""
 import json, sys
 from pathlib import Path
@@ -104,6 +105,24 @@ for dt, nb in ((torch.float32, 4), (torch.float64, 8)):
     n_out = n_chain * 10 * n_frame * 7
     report(f"pchip_kernel ({str(dt).split('.')[1]}, x10 upsampling of the angles tensor)", timeit(lambda: engine.pchip_resample(a, 0.01, 0.001), reps=5),
            (angles.numel() + n_out) * nb, n_out, "samples")
-    del a
+    # backward: series + grad_out in, grad_in out ((m + 2 n) width values per block row)
+    g_out = torch.randn((n_chain, 10 * n_frame, 7), device="cuda", generator=g).to(dt)
+    report(f"pchip_backward_kernel ({str(dt).split('.')[1]})", timeit(lambda: engine.pchip_resample_backward(a, g_out, 0.01, 0.001), reps=5),
+           (2 * angles.numel() + n_out) * nb, n_out, "samples")
+    a_req = a.clone().requires_grad_()
+    report(f"pchip_resample + backward through autograd ({str(dt).split('.')[1]}, kernels)",
+           timeit(lambda: torch.autograd.grad(engine.pchip_resample(a_req, 0.01, 0.001), [a_req], g_out), reps=5),
+           (3 * angles.numel() + 2 * n_out) * nb, n_out, "samples")
+    del g_out, a_req, a
+# what a user would write without the kernels: the float32 torch-ops model (tests/model_pchip.py) + torch autograd VJP,
+# on the (series, sample) layout; bytes: those of the two kernels
+sys.path.insert(0, str(ROOT / "tests"))
+import model_pchip
+a_t = angles.permute(0, 2, 1).reshape(-1, n_frame).contiguous().requires_grad_()
+g_t = torch.randn((a_t.shape[0], 10 * n_frame), device="cuda", generator=g)
+report("float32 torch-ops pchip + torch autograd VJP (reference point)",
+       timeit(lambda: torch.autograd.grad(model_pchip.resample(a_t, 0.01, 0.001), [a_t], g_t), reps=3),
+       (3 * angles.numel() + 2 * n_chain * 10 * n_frame * 7) * 4, n_chain * 10 * n_frame * 7, "samples")
+del a_t, g_t
 x = torch.empty(1 << 28, device="cuda"); y = torch.empty_like(x)
 report("torch copy (reference point)", timeit(lambda: y.copy_(x)), 2 * x.numel() * 4, x.numel(), "elements")

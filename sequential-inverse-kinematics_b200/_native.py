@@ -12,7 +12,7 @@ import numpy as np
 _HERE = Path(__file__).resolve().parent
 LIB_PATH = _HERE / "csrc" / "libseqik_sm100.so"
 
-ABI_VERSION = 10
+ABI_VERSION = 11
 CHAIN_PARAM_FLOATS = 32
 FLAG_ESCAPE = 1 << 4
 FLAG_SKIP_CONFIRM = 1 << 5
@@ -40,6 +40,8 @@ _SIGNATURES = {
                                            _vp, _vp, _i64, _i64, _u32, _vp]),
     "seqik_pchip_resample_f32": (_int, [_vp, _vp, _i64, _i64, _i64, _i64, ctypes.c_double, ctypes.c_double, _vp]),
     "seqik_pchip_resample_f64": (_int, [_vp, _vp, _i64, _i64, _i64, _i64, ctypes.c_double, ctypes.c_double, _vp]),
+    "seqik_pchip_resample_backward_f32": (_int, [_vp, _vp, _vp, _i64, _i64, _i64, _i64, ctypes.c_double, ctypes.c_double, _vp]),
+    "seqik_pchip_resample_backward_f64": (_int, [_vp, _vp, _vp, _i64, _i64, _i64, _i64, ctypes.c_double, ctypes.c_double, _vp]),
     "seqik_memcpy2d_async": (_int, [_vp, _i64, _vp, _i64, _i64, _i64, _int, _vp]),
     "seqik_fk_expand_host_f32": (_int, [_vp, _i64, _i64, _vp, _i64, _i64, _vp, _i64, _i64, _i64, _i64, _i64, _int]),
     "seqik_fk_f32": (_int, [_vp, _vp, _i64, _vp, _vp, _i64, _i64, _vp]),

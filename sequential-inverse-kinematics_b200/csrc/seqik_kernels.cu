@@ -21,6 +21,7 @@
 #include "seqik_common.h"
 #include "seqik_core.cuh"
 #include "seqik_head.cuh"
+#include "seqik_pchip.cuh"
 #include "seqik_stream.cuh"
 
 using namespace seqik;
@@ -1199,20 +1200,6 @@ extern "C" int seqik_head_apply_f32(const float* head, const float* affine, floa
 // about the left knot, and -- because the new grid runs past the last sample -- the last piece extrapolated.
 // One thread per output sample; `width` interleaved channels ([block][sample][width], e.g. the 7 DOFs of an angles
 // tensor) so that loads and stores of neighbouring threads are contiguous.  HBM-bound: (n + m) * width values per block.
-__device__ __forceinline__ float pchip_div(float a, float b) { return __fdividef(a, b); }     // <= 2 ulp; |b| < 2^126 here
-__device__ __forceinline__ double pchip_div(double a, double b) { return a / b; }
-template <typename T> __device__ __forceinline__ T pchip_sign(T v) { return (T)((v > T(0)) - (v < T(0))); }
-template <typename T> __device__ __forceinline__ T pchip_edge(T h0, T h1, T m0, T m1) {      // scipy PchipInterpolator._edge_case
-    T d = pchip_div((T(2) * h0 + h1) * m0 - h0 * m1, h0 + h1);
-    if (pchip_sign(d) != pchip_sign(m0)) d = T(0);
-    else if (pchip_sign(m0) != pchip_sign(m1) && fabs(d) > T(3) * fabs(m0)) d = T(3) * m0;
-    return d;
-}
-template <typename T> __device__ __forceinline__ T pchip_inner(T ma, T mb) {                 // _find_derivatives, interior point
-    // uniform grid: w1 = w2 = 3 h, so 1 / ((w1 / ma + w2 / mb) / (w1 + w2)) is the harmonic mean 2 ma mb / (ma + mb)
-    if (pchip_sign(ma) != pchip_sign(mb) || ma == T(0) || mb == T(0)) return T(0);
-    return pchip_div(T(2) * ma * mb, ma + mb);
-}
 // W = compile-time channel count (1 or 7: index arithmetic by multiply-shift), 0 = run-time `width` (<= 256).
 // One thread per (interval k, channel j): the derivatives and the cubic's coefficients are computed once per interval and
 // every sample of the new grid that falls into it is evaluated from them (10 samples per interval for 100 Hz -> 1 kHz);
@@ -1220,7 +1207,6 @@ template <typename T> __device__ __forceinline__ T pchip_inner(T ma, T mb) {    
 // CONTIGUOUS range of the output, which it assembles in shared memory and writes with coalesced (128-bit) stores; ranges
 // too long for the buffer (extreme up-sampling) are stored directly.  grid.x tiles the n - 1 intervals of one block row,
 // grid.y strides over the block rows (the FP64 interval bounds are computed once per thread): no 64-bit division.
-constexpr int PCHIP_STAGE_BYTES = 32768;
 template <typename T, int W>
 __global__ void __launch_bounds__(256) pchip_kernel(const T* __restrict__ in, T* __restrict__ out, int64_t n_block, int n,
                                                     int m, int width_rt, double ts, double new_ts, double inv_new_ts) {
@@ -1237,13 +1223,7 @@ __global__ void __launch_bounds__(256) pchip_kernel(const T* __restrict__ in, T*
     const double xk = (double)k * ts, xk1 = (double)(k + 1) * ts;
     int u_lo = 0, u_hi = 0;
     if (active) {
-        u_lo = (int)ceil(xk * inv_new_ts); u_hi = (int)ceil(xk1 * inv_new_ts);
-        while (u_lo > 0 && (double)(u_lo - 1) * new_ts >= xk) --u_lo;
-        while ((double)u_lo * new_ts < xk) ++u_lo;
-        while (u_hi > 0 && (double)(u_hi - 1) * new_ts >= xk1) --u_hi;
-        while ((double)u_hi * new_ts < xk1) ++u_hi;
-        if (k == n - 2) u_hi = m;                               // the last piece is extrapolated over the rest of the grid
-        u_hi = min(u_hi, m); u_lo = min(u_lo, u_hi);
+        pchip_bounds(k, n, m, xk, xk1, new_ts, inv_new_ts, u_lo, u_hi);
         if (j == 0 && k == k0) s_first = u_lo;
         if (j == 0 && k == k1) s_end = u_hi;
     }

@@ -491,10 +491,30 @@ def pchip_resample(series, original_ts: float, new_ts: float):
     series on the device: ``series`` (n_block, n, width) -- e.g. an angles tensor (n_chain, n_frame, 7) -- or (n_series, n);
     float32 or float64.  Returns the same layout with ``m = len(np.arange(0, n * original_ts, new_ts))`` samples.
     Like the reference's retry (utils.py:343-347: ``signal[np.isinf(signal)] = 0; signal[-1] = 0`` on the WHOLE array of one
-    call), +-inf samples are zeroed and, in every block that held one, the last sample of ALL its channels; NaN raises."""
-    import numpy as np
+    call), +-inf samples are zeroed and, in every block that held one, the last sample of ALL its channels; NaN raises.
+
+    Differentiable: when grad mode is on and ``series`` requires grad, the result carries a ``grad_fn`` whose backward is
+    the ``seqik_pchip_resample_backward`` kernel (see ``pchip_resample_backward``); the samples the forward replaced by 0
+    get gradient 0.  First derivatives only: a second backward raises.  Without grad the call is the plain kernel launch."""
     torch = N.require_cuda()
+    if torch.is_grad_enabled() and isinstance(series, torch.Tensor) and series.requires_grad:
+        return _pchip_function().apply(series, original_ts, new_ts)
+    x, flat, m, _ = _pchip_inputs(torch, series, original_ts, new_ts)
+    n_block, n, width = (int(v) for v in x.shape)
     lib = N.load_library()
+    out = torch.empty((n_block, m, width), dtype=x.dtype, device=x.device)
+    fn = lib.seqik_pchip_resample_f32 if x.dtype == torch.float32 else lib.seqik_pchip_resample_f64
+    with torch.cuda.device(x.device):
+        rc = fn(x.data_ptr(), out.data_ptr(), n_block, n, m, width, float(original_ts), float(new_ts),
+                N.stream_ptr(torch, x.device))
+    N.check(rc, "seqik_pchip_resample")
+    return out.squeeze(-1) if flat else out
+
+
+def _pchip_inputs(torch, series, original_ts, new_ts):
+    """Checks of the resampler's input -> (the series as the kernel reads it (n_block, n, width), whether it was 2-D, m,
+    the mask of the samples replaced by 0 or None)."""
+    import numpy as np
     if not isinstance(series, torch.Tensor) or not series.is_cuda:
         raise N.SeqIKNativeError("series must be a CUDA tensor (there is no CPU path)")
     if series.dtype not in (torch.float32, torch.float64):
@@ -502,15 +522,17 @@ def pchip_resample(series, original_ts: float, new_ts: float):
     if series.dim() not in (2, 3):
         raise ValueError("series must be (n_series, n) or (n_block, n, width)")
     flat = series.dim() == 2
-    x = series.unsqueeze(-1) if flat else series
+    x = series.detach()
+    x = x.unsqueeze(-1) if flat else x
     if not x.is_contiguous():
         raise ValueError("series must be contiguous")
-    n_block, n, width = (int(v) for v in x.shape)
+    n = int(x.shape[1])
     if n < 2:
         raise ValueError("at least 2 samples are needed")
     if not (original_ts > 0 and new_ts > 0):
         raise ValueError("time steps must be positive")
     m = int(np.ceil((n * original_ts) / new_ts))                # length of np.arange(0, n * original_ts, new_ts)
+    zeroed = None
     # one read-only pass; NaN propagates, +-inf shows up as an extreme (an empty batch has nothing to check)
     if x.numel() and not bool(torch.isfinite(torch.stack(torch.aminmax(x))).all()):
         finite = torch.isfinite(x)
@@ -519,10 +541,60 @@ def pchip_resample(series, original_ts: float, new_ts: float):
         x = torch.where(finite, x, torch.zeros_like(x))
         hit = (~finite).any(dim=1).any(dim=1, keepdim=True)       # (n_block, 1): blocks (= one reference call) that held an inf
         x[:, -1, :] = torch.where(hit, torch.zeros_like(x[:, -1, :]), x[:, -1, :])
-    out = torch.empty((n_block, m, width), dtype=x.dtype, device=x.device)
-    fn = lib.seqik_pchip_resample_f32 if x.dtype == torch.float32 else lib.seqik_pchip_resample_f64
+        zeroed = ~finite
+        zeroed[:, -1, :] |= hit
+    return x, flat, m, zeroed
+
+
+def pchip_resample_backward(series, grad_out, original_ts: float, new_ts: float):
+    """Vector-Jacobian product of ``pchip_resample``: ``grad_out`` = dL/dout in the layout of the resampled series ->
+    dL/dseries in the layout and dtype of ``series``, (n_series, n) or (n_block, n, width).  The gradient is taken at the
+    values the forward resampled; the samples it replaced by 0 (+-inf, and the last sample of a block that held one) get
+    gradient 0.  The float summation order is fixed (include/seqik.h), so the result is deterministic."""
+    torch = N.require_cuda()
+    x, flat, m, zeroed = _pchip_inputs(torch, series, original_ts, new_ts)
+    n_block, n, width = (int(v) for v in x.shape)
+    if not isinstance(grad_out, torch.Tensor) or grad_out.device != x.device or grad_out.dtype != x.dtype:
+        raise ValueError(f"grad_out must be a {x.dtype} tensor on {x.device}")
+    want = (n_block, m) if flat else (n_block, m, width)
+    if tuple(grad_out.shape) != want:
+        raise ValueError(f"grad_out must be {want}, got {tuple(grad_out.shape)}")
+    g = grad_out.detach().reshape(n_block, m, width).contiguous()
+    lib = N.load_library()
+    grad = torch.empty_like(x)
+    fn = lib.seqik_pchip_resample_backward_f32 if x.dtype == torch.float32 else lib.seqik_pchip_resample_backward_f64
     with torch.cuda.device(x.device):
-        rc = fn(x.data_ptr(), out.data_ptr(), n_block, n, m, width, float(original_ts), float(new_ts),
+        rc = fn(x.data_ptr(), g.data_ptr(), grad.data_ptr(), n_block, n, m, width, float(original_ts), float(new_ts),
                 N.stream_ptr(torch, x.device))
-    N.check(rc, "seqik_pchip_resample")
-    return out.squeeze(-1) if flat else out
+    N.check(rc, "seqik_pchip_resample_backward")
+    if zeroed is not None:
+        grad.masked_fill_(zeroed, 0)
+    return grad.squeeze(-1) if flat else grad
+
+
+_PCHIP_FUNCTION = None
+
+
+def _pchip_function():
+    """The torch.autograd.Function of pchip_resample (built on first use: torch is imported lazily)."""
+    global _PCHIP_FUNCTION
+    if _PCHIP_FUNCTION is not None:
+        return _PCHIP_FUNCTION
+    import torch
+    from torch.autograd.function import once_differentiable
+
+    class PchipResample(torch.autograd.Function):
+        @staticmethod
+        def forward(ctx, series, original_ts, new_ts):
+            ctx.save_for_backward(series)
+            ctx.steps = (original_ts, new_ts)
+            return pchip_resample(series, original_ts, new_ts)
+
+        @staticmethod
+        @once_differentiable
+        def backward(ctx, grad_out):
+            series, = ctx.saved_tensors
+            return pchip_resample_backward(series, grad_out, *ctx.steps), None, None
+
+    _PCHIP_FUNCTION = PchipResample
+    return _PCHIP_FUNCTION
