@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define SEQIK_ABI_VERSION 11  /* 11: seqik_pchip_resample_backward_f32/_f64; 10: seqik_head_angles_backward_f32; 9: seqik_fk_backward_f32; 8: seqik_origin_rows_f32; 7: seqik_leg_affine_from_pose_f32; 6: schedule 3 (frame-parallel blocks), seqik_fk_expand_host_f32; 5: solver flag bits 6-7, phase periods in bits 21-27 */
+#define SEQIK_ABI_VERSION 12  /* 12: seqik_align_apply_backward_f32, seqik_leg_affine_backward_f32; 11: seqik_pchip_resample_backward_f32/_f64; 10: seqik_head_angles_backward_f32; 9: seqik_fk_backward_f32; 8: seqik_origin_rows_f32; 7: seqik_leg_affine_from_pose_f32; 6: schedule 3 (frame-parallel blocks), seqik_fk_expand_host_f32; 5: solver flag bits 6-7, phase periods in bits 21-27 */
 #define SEQIK_OK 0
 #define SEQIK_EINVAL (-1)
 #define SEQIK_ECUDA (-3)
@@ -295,6 +295,47 @@ int seqik_leg_affine_from_pose_f32(const float* pose, int64_t pose_chain_stride,
  * out[:,0] = template, out[:,i] = (pose[:,i] - fixed) * scale + template.   affine [n_chain][8] as above. */
 int seqik_align_apply_f32(const float* pose, int64_t pose_chain_stride, int64_t pose_frame_stride,
                           const float* affine, float* out, int64_t n_chain, int64_t n_frame, void* stream);
+
+/* Backward of seqik_align_apply_f32 (vector-Jacobian product), given grad_out = dL/dout.  New in this library: the reference
+ * has no gradients, so this replaces nothing in it.
+ *   pose, strides, affine: as for seqik_align_apply_f32;  grad_out [n_chain][n_frame][5][3] in (dense)
+ *   grad_pose            NULL (skip), or [n_chain][n_frame][5][3] out (dense): 0 for key point 0 (it is replaced by the
+ *                        template), aff[3] * grad_out for key points 1..4 (one float32 multiplication)
+ *   grad_affine_partial  NULL (skip), or [n_chain][n_frame][8] out (dense): each leg-frame's contribution to dL/daffine (the
+ *                        caller sums over frames).  With g_i = grad_out[c][t][i], d_i = ((p_ix - a0) g_ix + (p_iy - a1) g_iy)
+ *                        + (p_iz - a2) g_iz and, per coordinate, S = ((g_1 + g_2) + g_3) + g_4, in float32 and in this order:
+ *                          [0..2] = -(a3 S),  [3] = ((d_1 + d_2) + d_3) + d_4,  [4..6] = g_0 + S,  [7] = 0
+ * Deterministic (no atomics); the bits do not depend on the launch path (dense and 16-byte aligned buffers stream through
+ * the TMA tile pipeline, anything else through a plain kernel).  Sizes, NULL and stride errors are the forward's. */
+int seqik_align_apply_backward_f32(const float* pose, int64_t pose_chain_stride, int64_t pose_frame_stride,
+                                   const float* affine, const float* grad_out, float* grad_pose, float* grad_affine_partial,
+                                   int64_t n_chain, int64_t n_frame, void* stream);
+
+/* Backward of seqik_leg_affine_from_pose_f32 (vector-Jacobian product), given grad_affine = dL/daffine [n_chain][8].  New in
+ * this library.  With H = grad_affine[c], m_s the seven mid-quantiles (coxa x, y, z, the four segment lengths), len = (m_3 +
+ * m_4) + m_5 [+ m_6 with include_claw] and scale = affine[c][3]:
+ *   grad_consts  NULL (skip), or [n_chain][4] out = (H4, H5, H6, H3 / len)
+ *   grad_pose    [n_chain][n_frame][5][3] (dense, required): the statistics' contributions are ADDED to it, so a caller
+ *                passes zeros or the output of seqik_align_apply_backward_f32.  dL/dm_s = H_s for the coxa series,
+ *                -(H3 scale) / len for every length in len (the tarsus only with include_claw).  A mid-quantile
+ *                0.5 ((v0 + (v1 - v0) f45) + (v2 + (v3 - v2) f55)) passes dL/dm to its order statistics with the weights
+ *                0.5 (1 - f45), 0.5 f45, 0.5 (1 - f55), 0.5 f55 (ranks and weights of seqik_mid_quantile_f32; coinciding
+ *                ranks add).  The order statistic of rank r sits in frame t_r; a coxa series sends its share to
+ *                pose[t_r][0][coordinate], a length series j sends +share s / |s| to key point j+1 and -share s / |s| to key
+ *                point j of frame t_r (s the segment vector; a squared length of exactly 0 contributes 0).
+ *   Tie rule: keys are the forward's order keys (-0 below +0), the lengths compared on their float32 SQUARED lengths
+ *   (dx dx + dy dy) + dz dz on every path; t_r is the (r - #{keys < key_r})-th frame, in ascending frame order, among the
+ *   frames whose key equals key_r: argsort(keys, stable)[r].
+ *   The mid-quantiles and len are recomputed from the selected keys with the forward's float32 arithmetic.  One thread per
+ *   chain adds the contributions in a fixed order (series 0..6, rank position 0..3; end point before base point), so the
+ *   result is deterministic.  Error bound against the float64 VJP at the same frames (u = 2^-24): per float of grad_pose
+ *   64 u N A, N the contributions it receives and A the sum of their absolute values; 16 u |dL/dconsts| for grad_consts.
+ *   scratch: NULL for recordings of up to 1024 frames (one CTA per chain), else n_chain * 7 * (n_frame + 12) 32-bit words.
+ * Sizes, NULL, stride and empty-recording errors are the forward's. */
+int seqik_leg_affine_backward_f32(const float* pose, int64_t pose_chain_stride, int64_t pose_frame_stride,
+                                  const float* consts, int include_claw, const float* affine, const float* grad_affine,
+                                  float* grad_pose, float* grad_consts, uint32_t* scratch,
+                                  int64_t n_chain, int64_t n_frame, void* stream);
 
 /* Antenna series of AlignPose.align_head (alignment.py:489-555).
  *   head [n_trial][n_frame][2][3] (base, tip), thorax [n_trial][n_frame][n_thorax_kp][3] (first and last

@@ -3,7 +3,8 @@
 Algorithmic bytes per unit (DESIGN.md 5.3): fk 28+12+108 B/leg-frame (origin per frame), fk backward 28+108 in and 28+12
 (+16 with the lengths) out, head 48+28 B/frame (+12 with a
 per-frame neck), head backward 48+28 in and 48+12 out, pchip n+m values per block row and channel, pchip backward n+m in
-and n out, align_apply 60+60 B/leg-frame, leg_series 60 in + 28 out, mid_quantile 4 B/element read (4 ranks x
+and n out, align_apply 60+60 B/leg-frame, align_apply backward 60+60 in and 60+32 out, leg_affine backward 60 B read twice
+(fused path; the long path writes 28 B of keys and reads them in the select's four passes and the frame sweep), leg_series 60 in + 28 out, mid_quantile 4 B/element read (4 ranks x
 4 radix passes re-read the series: from L2 when it fits)."""
 import json, sys
 from pathlib import Path
@@ -75,6 +76,50 @@ rec = base.repeat((n_chain + base.shape[0] - 1) // base.shape[0], 1, 1, 1)[:n_ch
 report("leg_affine fused, recording-like key points", timeit(lambda: engine.leg_affine(rec, consts)), lf * 60 + n_chain * 32, lf, "leg-frames")
 report("leg_affine fused, normal-random key points (wide-range series)", timeit(lambda: engine.leg_affine(pose, consts)), lf * 60 + n_chain * 32, lf, "leg-frames")
 report("leg_affine three-kernel path (series + select + affine), recording-like", timeit(lambda: engine.leg_affine_unfused(rec, consts)), lf * (60 + 28 + 28), lf, "leg-frames")
+# alignment backward: apply backward (pose + dL/dout in, dL/dpose + per-leg-frame dL/daffine rows out, + the frame sum), the
+# statistics backward on the fused path (key points read twice, 28 scattered contributions per chain), forward + backward
+# through autograd, and the same VJP through torch autograd of the alignment in float32 torch ops with torch.quantile
+aff_rec = engine.leg_affine(rec, consts)
+g_al = torch.randn(rec.shape, device="cuda", generator=g)
+h_al = torch.randn((n_chain, 8), device="cuda", generator=g)
+gp_buf = torch.zeros_like(rec)
+report("align_apply_backward (tile kernel + frame sum)", timeit(lambda: engine.align_apply_backward(rec, aff_rec, g_al)), lf * (60 + 60 + 60 + 32), lf, "leg-frames")
+report("leg_affine_backward fused, recording-like", timeit(lambda: engine.leg_affine_backward(rec, consts, aff_rec, h_al, grad_pose=gp_buf)),
+       lf * 120 + n_chain * 32, lf, "leg-frames")
+rec_req = rec.clone().requires_grad_()
+report("align_apply(leg_affine) + backward through autograd (kernels)",
+       timeit(lambda: torch.autograd.grad(engine.align_apply(rec_req, engine.leg_affine(rec_req, consts)), [rec_req], g_al)),
+       lf * (60 + 60 + 60 + 60 + 60 + 32 + 120 + 60), lf, "leg-frames")
+
+
+def torch_align(p, k):
+    seg = p[:, :, 1:] - p[:, :, :-1]
+    series = torch.cat([p[:, :, 0], torch.linalg.vector_norm(seg, dim=-1)], dim=-1)                     # (chain, frame, 7)
+    m = torch.quantile(series, torch.tensor([0.45, 0.55], device=p.device), dim=1).mean(0)
+    scale = k[:, 3] / ((m[:, 3] + m[:, 4]) + m[:, 5])
+    moved = (p[:, :, 1:] - m[:, None, None, :3]) * scale[:, None, None, None] + k[:, None, None, :3]
+    return torch.cat([k[:, None, None, :3].expand(-1, p.shape[1], 1, 3), moved], dim=2)
+
+
+def torch_align_vjp():                                             # torch.quantile takes at most 2^24 values per call
+    for c0 in range(0, n_chain, 1000):
+        torch.autograd.grad(torch_align(rec_req[c0:c0 + 1000], consts[c0:c0 + 1000]), [rec_req], g_al[c0:c0 + 1000])
+
+
+report("float32 torch-ops alignment (torch.quantile) + torch autograd VJP (reference point)", timeit(torch_align_vjp, reps=3),
+       lf * (60 + 60 + 60 + 60 + 60 + 32 + 120 + 60), lf, "leg-frames")
+del g_al, gp_buf, rec_req, aff_rec
+# the long path: 600 chains x 100 000 frames (series through scratch): the recording-like chains repeated, with 1 um noise
+lp = rec[:600].repeat(1, 100, 1, 1) + 1e-3 * torch.randn((600, 100 * n_frame, 5, 3), device="cuda", generator=g)
+lc = consts[:lp.shape[0]].contiguous()
+lf_long = lp.shape[0] * lp.shape[1]
+aff_long = engine.leg_affine(lp, lc)
+h_long = torch.randn((lp.shape[0], 8), device="cuda", generator=g)
+gp_long = torch.zeros_like(lp)
+report("leg_affine long path (600 x 100 000)", timeit(lambda: engine.leg_affine(lp, lc), reps=5), lf_long * (60 + 28 + 28), lf_long, "leg-frames")
+report("leg_affine_backward long path (600 x 100 000): keys + select + frames + scatter", timeit(lambda: engine.leg_affine_backward(lp, lc, aff_long, h_long, grad_pose=gp_long), reps=5),
+       lf_long * (60 + 28 + 4 * 28 + 28), lf_long, "leg-frames")
+del lp, gp_long
 del base
 nf = n_trial * n_frame * 6
 r = torch.randn((n_trial, 6 * n_frame, 2, 3), device="cuda", generator=g); l = torch.randn((n_trial, 6 * n_frame, 2, 3), device="cuda", generator=g)

@@ -12,7 +12,7 @@ import numpy as np
 _HERE = Path(__file__).resolve().parent
 LIB_PATH = _HERE / "csrc" / "libseqik_sm100.so"
 
-ABI_VERSION = 11
+ABI_VERSION = 12
 CHAIN_PARAM_FLOATS = 32
 FLAG_ESCAPE = 1 << 4
 FLAG_SKIP_CONFIRM = 1 << 5
@@ -54,6 +54,8 @@ _SIGNATURES = {
     "seqik_origin_rows_f32": (_int, [_vp, _i64, _i64, _vp, _i64, _i64, _i64, _i64, _vp]),
     "seqik_leg_affine_from_pose_f32": (_int, [_vp, _i64, _i64, _vp, _int, _vp, _vp, _i64, _i64, _vp]),
     "seqik_align_apply_f32": (_int, [_vp, _i64, _i64, _vp, _vp, _i64, _i64, _vp]),
+    "seqik_align_apply_backward_f32": (_int, [_vp, _i64, _i64, _vp, _vp, _vp, _vp, _i64, _i64, _vp]),
+    "seqik_leg_affine_backward_f32": (_int, [_vp, _i64, _i64, _vp, _int, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _vp]),
     "seqik_head_series_f32": (_int, [_vp, _vp, _i64, _f32, _vp, _vp, _i64, _i64, _vp]),
     "seqik_head_series_f64": (_int, [_vp, _vp, _i64, ctypes.c_double, _vp, _vp, _i64, _i64, _vp]),
     "seqik_head_affine_f32": (_int, [_vp, _vp, _vp, _i64, _vp]),

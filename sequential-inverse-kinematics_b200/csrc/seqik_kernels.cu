@@ -22,6 +22,7 @@
 #include "seqik_core.cuh"
 #include "seqik_head.cuh"
 #include "seqik_pchip.cuh"
+#include "seqik_select.cuh"
 #include "seqik_stream.cuh"
 
 using namespace seqik;
@@ -362,29 +363,9 @@ extern "C" int seqik_leg_series_f32(const float* pose, int64_t pose_chain_stride
     return check_launch("seqik_leg_series_f32");
 }
 
-// Order statistic by 4-pass MSB radix select on order-preserving keys; one block per (series, rank).
-__device__ __forceinline__ uint32_t order_key(float f) {
-    // The bits go through an opaque move.  From __float_as_uint(f), the compiler turned `u | 0x80000000` into a float
-    // negation of |f| (FADD -|f|, -0), which makes a NaN the canonical 0x7fffffff: a key just below +0's, inside any range
-    // that straddles zero (the long kernel's NaN padding of its float4 sweeps included).
-    uint32_t u;
-    asm("mov.b32 %0, %1;" : "=r"(u) : "f"(f));
-    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-__device__ __forceinline__ float key_value(uint32_t k) {
-    return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k);
-}
-
+// Order statistic by 4-pass MSB radix select on order-preserving keys (order_key, seqik_select.cuh); one block per (series, rank).
 constexpr int SEL_BLOCK = 256;
 constexpr int SEL_CACHE = 8192;             // order keys of a series cached in shared memory up to this length
-
-// ranks of numpy.quantile(..., method="linear") at q = 0.45 and 0.55: floor(q (n-1)) and the next one
-__device__ __forceinline__ void quantile_pos(double q, int64_t n, int64_t& lo, float& frac) {
-    const double v = q * (double)(n - 1);
-    lo = (int64_t)floor(v);
-    if (lo > n - 1) lo = n - 1;
-    frac = (float)(v - (double)lo);
-}
 
 // One block per series: the four order statistics (two neighbours of each of the 0.45 / 0.55 quantile positions)
 // are found together by a 4-pass MSB radix select -- per pass one sweep over the series (from shared memory when it
@@ -631,19 +612,8 @@ __device__ void warp_select4(uint32_t* __restrict__ key, int n, unsigned int* ra
     }
 }
 
-// the four ranks of the mid-quantile of the m smallest keys, and the interpolation weights (numpy "linear").  The ranks
-// come out non-decreasing, as warp_select4 and the long kernel's bin search require: for m = 2, 4, 6, 8, 10 both positions
-// have the same lower neighbour (lo45 == lo55), and lo, lo + 1, lo, lo + 1 is selected as lo, lo, lo + 1, lo + 1.  The
-// return value says so; mid_quantile_value puts the middle two back.
-__device__ __forceinline__ bool mid_quantile_ranks(int64_t m, unsigned int* rank, float& f45, float& f55) {
-    int64_t lo45, lo55;
-    quantile_pos(0.45, m, lo45, f45); quantile_pos(0.55, m, lo55, f55);
-#pragma unroll
-    for (int k = 0; k < 4; ++k) { const int64_t r = (k < 2 ? lo45 : lo55) + (k & 1); rank[k] = (unsigned int)(r > m - 1 ? m - 1 : r); }
-    const bool swap = rank[1] > rank[2];
-    if (swap) { const unsigned int t = rank[1]; rank[1] = rank[2]; rank[2] = t; }
-    return swap;
-}
+
+// the forward's mid-quantile of the four selected keys (ranks and swap: mid_quantile_ranks, seqik_select.cuh)
 __device__ __forceinline__ float mid_quantile_value(const uint32_t* val, float f45, float f55, bool swap) {
     const float a0 = key_value(val[0]), a1 = key_value(val[swap ? 2 : 1]), b0 = key_value(val[swap ? 1 : 2]), b1 = key_value(val[3]);
     const float q0 = a0 + (a1 - a0) * f45, q1 = b0 + (b1 - b0) * f55;

@@ -389,8 +389,30 @@ def mid_quantile(series, counts=None):
 
 def leg_affine(pose, consts, include_claw: bool = False):
     """AlignPose.align_leg statistics: pose (n_chain, n_frame, 5, 3), consts (n_chain, 4) = template coxa xyz + model
-    length -> affine (n_chain, 8) = (fixed_coxa xyz, scale, template xyz, 0)."""
+    length -> affine (n_chain, 8) = (fixed_coxa xyz, scale, template xyz, 0).
+
+    Differentiable: when grad mode is on and ``pose`` or ``consts`` requires grad, the result carries a ``grad_fn`` whose
+    backward is the ``seqik_leg_affine_backward_f32`` kernel (see ``leg_affine_backward``): each mid-quantile passes its
+    gradient to the key points of the frames that hold its four order statistics (ties: the first frames in frame order,
+    include/seqik.h).  First derivatives only: a second backward raises.  Without inputs that require grad the call is the
+    plain kernel launch."""
     torch = N.require_cuda()
+    if torch.is_grad_enabled() and any(isinstance(t, torch.Tensor) and t.requires_grad for t in (pose, consts)):
+        return _align_functions()[0].apply(pose, consts, bool(include_claw))
+    return _leg_affine(torch, pose, consts, include_claw)
+
+
+def _leg_affine_inputs(pose, consts):
+    pose = _check(pose, "pose", (5, 3))
+    if pose.dim() != 4:
+        raise ValueError(f"pose must be (n_chain, n_frame, 5, 3), got {tuple(pose.shape)}")
+    consts = _check(consts, "consts", (4,))
+    if consts.dim() != 2 or consts.shape[0] != pose.shape[0]:
+        raise ValueError("consts must have one row per chain")
+    return int(pose.shape[0]), int(pose.shape[1])
+
+
+def _leg_affine(torch, pose, consts, include_claw):
     lib = N.load_library()
     pose = _check(pose, "pose", (5, 3))
     n_chain, n_frame = int(pose.shape[0]), int(pose.shape[1])
@@ -406,6 +428,35 @@ def leg_affine(pose, consts, include_claw: bool = False):
                                                    N.ptr(scratch), N.ptr(affine), n_chain, n_frame, N.stream_ptr(torch, dev)),
                 "seqik_leg_affine_from_pose_f32")
     return affine
+
+
+def leg_affine_backward(pose, consts, affine, grad_affine, include_claw: bool = False, grad_pose=None):
+    """Vector-Jacobian product of ``leg_affine``: grad_affine (n_chain, 8) = dL/daffine -> (grad_pose (n_chain, n_frame, 5, 3),
+    grad_consts (n_chain, 4)).  ``affine`` is the forward's result.  The statistics' contributions are ADDED into
+    ``grad_pose`` when it is given (e.g. the output of ``align_apply_backward``; updated in place), else into zeros.  The
+    frames, the tie rule and the float summation order are those of include/seqik.h: the result is deterministic."""
+    torch = N.require_cuda()
+    lib = N.load_library()
+    n_chain, n_frame = _leg_affine_inputs(pose, consts)
+    _check(affine, "affine", (8,))
+    grad_affine = _check(grad_affine, "grad_affine", (8,))
+    if tuple(affine.shape) != (n_chain, 8) or tuple(grad_affine.shape) != (n_chain, 8):
+        raise ValueError(f"affine and grad_affine must be ({n_chain}, 8)")
+    dev = pose.device
+    if grad_pose is None:
+        grad_pose = torch.zeros_like(pose)
+    else:
+        _check(grad_pose, "grad_pose", (5, 3))
+        if grad_pose.shape != pose.shape:
+            raise ValueError(f"grad_pose must be {tuple(pose.shape)}")
+    grad_consts = torch.empty((n_chain, 4), dtype=torch.float32, device=dev)
+    scratch = None if n_frame <= 1024 else torch.empty((n_chain * 7 * (n_frame + 12),), dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        rc = lib.seqik_leg_affine_backward_f32(N.ptr(pose), n_frame * 15, 15, N.ptr(consts), int(bool(include_claw)), N.ptr(affine),
+                                               N.ptr(grad_affine), N.ptr(grad_pose), N.ptr(grad_consts), N.ptr(scratch),
+                                               n_chain, n_frame, N.stream_ptr(torch, dev))
+    N.check(rc, "seqik_leg_affine_backward_f32")
+    return grad_pose, grad_consts
 
 
 def leg_affine_unfused(pose, consts, include_claw: bool = False):
@@ -430,8 +481,20 @@ def leg_affine_unfused(pose, consts, include_claw: bool = False):
 
 
 def align_apply(pose, affine):
-    """The affine map of align_leg as a standalone pass -> aligned pose (n_chain, n_frame, 5, 3)."""
+    """The affine map of align_leg as a standalone pass -> aligned pose (n_chain, n_frame, 5, 3).
+
+    Differentiable: when grad mode is on and ``pose`` or ``affine`` requires grad, the result carries a ``grad_fn`` whose
+    backward is the ``seqik_align_apply_backward_f32`` kernel (see ``align_apply_backward``).  Composed with ``leg_affine``
+    under autograd, ``align_apply(pose, leg_affine(pose, consts))`` gives the full gradient with respect to the raw key
+    points.  First derivatives only: a second backward raises.  Without inputs that require grad the call is the plain
+    kernel launch."""
     torch = N.require_cuda()
+    if torch.is_grad_enabled() and any(isinstance(t, torch.Tensor) and t.requires_grad for t in (pose, affine)):
+        return _align_functions()[1].apply(pose, affine)
+    return _align_apply(torch, pose, affine)
+
+
+def _align_apply(torch, pose, affine):
     lib = N.load_library()
     pose = _check(pose, "pose", (5, 3))
     affine = _check(affine, "affine", (8,))
@@ -442,6 +505,74 @@ def align_apply(pose, affine):
                                        N.stream_ptr(torch, pose.device))
     N.check(rc, "seqik_align_apply_f32")
     return out
+
+
+def align_apply_backward(pose, affine, grad_out, want_pose: bool = True, want_affine: bool = True):
+    """Vector-Jacobian product of ``align_apply``: grad_out (n_chain, n_frame, 5, 3) = dL/dout -> (grad_pose (n_chain,
+    n_frame, 5, 3) | None, grad_affine (n_chain, 8) | None).  grad_pose is aff[3] * grad_out with key point 0 at 0; grad_affine
+    is the sum over frames of the kernel's per-leg-frame rows (include/seqik.h)."""
+    torch = N.require_cuda()
+    lib = N.load_library()
+    pose = _check(pose, "pose", (5, 3))
+    affine = _check(affine, "affine", (8,))
+    if pose.dim() != 4 or affine.dim() != 2 or affine.shape[0] != pose.shape[0]:
+        raise ValueError("pose must be (n_chain, n_frame, 5, 3) and affine (n_chain, 8)")
+    grad_out = _check(grad_out, "grad_out", (5, 3))
+    if grad_out.shape != pose.shape:
+        raise ValueError(f"grad_out must be {tuple(pose.shape)}, got {tuple(grad_out.shape)}")
+    n_chain, n_frame = int(pose.shape[0]), int(pose.shape[1])
+    dev = pose.device
+    grad_pose = torch.empty_like(pose) if want_pose else None
+    part = torch.empty((n_chain, n_frame, 8), dtype=torch.float32, device=dev) if want_affine else None
+    with torch.cuda.device(dev):
+        rc = lib.seqik_align_apply_backward_f32(N.ptr(pose), n_frame * 15, 15, N.ptr(affine), N.ptr(grad_out), N.ptr(grad_pose),
+                                                N.ptr(part), n_chain, n_frame, N.stream_ptr(torch, dev))
+    N.check(rc, "seqik_align_apply_backward_f32")
+    return grad_pose, (part.sum(dim=1) if want_affine else None)
+
+
+_ALIGN_FUNCTIONS = None
+
+
+def _align_functions():
+    """The torch.autograd.Functions of leg_affine and align_apply (built on first use: torch is imported lazily)."""
+    global _ALIGN_FUNCTIONS
+    if _ALIGN_FUNCTIONS is not None:
+        return _ALIGN_FUNCTIONS
+    import torch
+    from torch.autograd.function import once_differentiable
+
+    class LegAffine(torch.autograd.Function):
+        @staticmethod
+        def forward(ctx, pose, consts, include_claw):
+            affine = _leg_affine(torch, pose, consts, include_claw)
+            ctx.save_for_backward(pose, consts, affine)
+            ctx.include_claw = include_claw
+            return affine
+
+        @staticmethod
+        @once_differentiable
+        def backward(ctx, grad_affine):
+            pose, consts, affine = ctx.saved_tensors
+            need_pose, need_consts = ctx.needs_input_grad[:2]
+            gp, gk = leg_affine_backward(pose, consts, affine, grad_affine.contiguous(), ctx.include_claw)
+            return (gp if need_pose else None), (gk if need_consts else None), None
+
+    class AlignApply(torch.autograd.Function):
+        @staticmethod
+        def forward(ctx, pose, affine):
+            ctx.save_for_backward(pose, affine)
+            return _align_apply(torch, pose, affine)
+
+        @staticmethod
+        @once_differentiable
+        def backward(ctx, grad_out):
+            pose, affine = ctx.saved_tensors
+            need_pose, need_affine = ctx.needs_input_grad
+            return align_apply_backward(pose, affine, grad_out.contiguous(), want_pose=need_pose, want_affine=need_affine)
+
+    _ALIGN_FUNCTIONS = (LegAffine, AlignApply)
+    return _ALIGN_FUNCTIONS
 
 
 def head_affine(head, thorax, consts, threshold: float = 5e-5):
