@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define SEQIK_ABI_VERSION 12  /* 12: seqik_align_apply_backward_f32, seqik_leg_affine_backward_f32; 11: seqik_pchip_resample_backward_f32/_f64; 10: seqik_head_angles_backward_f32; 9: seqik_fk_backward_f32; 8: seqik_origin_rows_f32; 7: seqik_leg_affine_from_pose_f32; 6: schedule 3 (frame-parallel blocks), seqik_fk_expand_host_f32; 5: solver flag bits 6-7, phase periods in bits 21-27 */
+#define SEQIK_ABI_VERSION 13  /* 13: seqik_head_apply_backward_f32, seqik_head_affine_backward_f32/_f64; 12: seqik_align_apply_backward_f32, seqik_leg_affine_backward_f32; 11: seqik_pchip_resample_backward_f32/_f64; 10: seqik_head_angles_backward_f32; 9: seqik_fk_backward_f32; 8: seqik_origin_rows_f32; 7: seqik_leg_affine_from_pose_f32; 6: schedule 3 (frame-parallel blocks), seqik_fk_expand_host_f32; 5: solver flag bits 6-7, phase periods in bits 21-27 */
 #define SEQIK_OK 0
 #define SEQIK_EINVAL (-1)
 #define SEQIK_ECUDA (-3)
@@ -359,6 +359,59 @@ int seqik_head_affine_f32(const float* stats, const float* consts, float* affine
  * (alignment.py:547-553).  head, out [n_trial][n_frame][2][3]. */
 int seqik_head_apply_f32(const float* head, const float* affine, float* out, int64_t n_trial, int64_t n_frame,
                          void* stream);
+
+/* Backward of seqik_head_apply_f32 (vector-Jacobian product), given grad_out = dL/dout.  New in this library: the reference
+ * has no gradients, so this replaces nothing in it.
+ *   head, affine: as for seqik_head_apply_f32;  grad_out [n_trial][n_frame][2][3] in.  With a = affine[trial], G_b and G_t
+ *   the frame's dL/d(aligned base) and dL/d(aligned tip), P_b = base - origin and P_t = tip - origin (the forward's float32
+ *   subtractions) and x . y = (x0 y0 + x1 y1) + x2 y2, in float32 and in this order:
+ *   grad_head            NULL (skip), or [n_trial][n_frame][2][3] out: (a3 G_b, a7 G_t), one float32 multiplication each
+ *                        (the affine contract of seqik_head_angles_backward_f32)
+ *   grad_affine_partial  NULL (skip), or [n_trial][n_frame][8] out: each frame's contribution to dL/daffine (the caller sums
+ *                        over frames): [0..2] = -((a3 G_b) + (a7 G_t)),  [3] = P_b . G_b,  [4..6] = G_b + G_t,  [7] = P_t . G_t
+ * All arrays dense.  Deterministic (no atomics); the bits do not depend on the launch path (16-byte aligned buffers stream
+ * through the TMA tile pipeline, anything else and the last partial tile through a plain kernel).  Size and NULL errors are
+ * the forward's. */
+int seqik_head_apply_backward_f32(const float* head, const float* affine, const float* grad_out, float* grad_head,
+                                  float* grad_affine_partial, int64_t n_trial, int64_t n_frame, void* stream);
+
+/* Backward of the head statistics -- seqik_head_series_f32/_f64, seqik_mid_quantile_f32 with the counts, seqik_head_affine_f32
+ * -- (vector-Jacobian product), given grad_affine = dL/daffine [n_trial][8].  New in this library.
+ *   head, thorax, n_thorax_kp: as for seqik_head_series_*, float32 (_f32) or float64 (_f64), dense
+ *   series, counts: what seqik_head_series_* wrote for the same inputs.  The stationary set is NOT decided again: it is
+ *           piecewise constant in the key points and is held fixed as the forward chose it
+ *   consts, affine: the forward's consts (checked, not read: the gradient does not depend on them) and result rows
+ *   grad_head    [n_trial][n_frame][2][3] (required), grad_thorax NULL (skip the thorax terms) or
+ *                [n_trial][n_frame][n_thorax_kp][3], in the input type: the statistics' contributions are ADDED to them
+ *   grad_consts  NULL (skip), or [n_trial][5] out
+ *   scratch: NULL for recordings of up to 1024 frames (one CTA per trial), else n_trial * 5 * (n_frame + 12) 32-bit words.
+ * With H = grad_affine[trial], a = affine[trial] and s_j the five mid-quantiles (base x, y, z, d, |tip - base|), recomputed
+ * from the selected keys with the forward's float32 arithmetic:
+ *   dL/ds = (H0, H1, H2, -(H3 a3) / s3, -(H7 a7) / s4),   grad_consts = (H4, H5, H6, H3 / s3, H7 / s4).
+ * Series j has m = counts[trial][j] values (the stationary frames for j = 0..3, every frame for j = 4); its mid-quantile
+ * passes dL/ds_j to its four order statistics with the weights of seqik_leg_affine_backward_f32 for m values, a share being
+ * weight * dL/ds_j in float32.  Tie rule: keys are the order keys of the float32 series values; the rank-r statistic sits in
+ * frame argsort(row keys, stable)[r].  The +inf padding sorts last and is never selected: finite inputs are the contract.
+ * With sh = the share rounded to the input type T, a frame t receives, in T:
+ *   j = 0..2: base[t][j] += sh
+ *   j = 3:    u = (b - 0.5 (t0 + t_last)) / d in float64 (b, t0 = thorax[t][0], t_last = thorax[t][k-1]; the arithmetic of
+ *             the series kernel) rounded to T, c = sh u:  base[t] += c, then thorax[t][0] -= 0.5 c, then thorax[t][k-1] -= 0.5 c
+ *             (for k = 1 both go to the same point)
+ *   j = 4:    v = (tip - base) / |tip - base| in float64 rounded to T, c = sh v:  tip[t] += c, then base[t] -= c
+ *   a distance or length of exactly 0 contributes 0; a series with m = 0 scatters nothing (its s_j is NaN, and so is the
+ *   grad_consts entry that divides by it).
+ * One thread per trial adds in a fixed order (series 0..4, sorted rank position 0..3, the points in the order above, x, y, z),
+ * so the result is deterministic.  Error bound against the float64 VJP at the same frames (u = 2^-24), in either type: per
+ * element of grad_head / grad_thorax 64 u N A, N the contributions it receives and A the sum of their absolute values;
+ * 16 u |dL/dconsts| for grad_consts.  Size, NULL and n_thorax_kp errors are the forward's; an empty recording is an error. */
+int seqik_head_affine_backward_f32(const float* head, const float* thorax, int64_t n_thorax_kp, const float* series,
+                                   const int32_t* counts, const float* consts, const float* affine, const float* grad_affine,
+                                   float* grad_head, float* grad_thorax, float* grad_consts, uint32_t* scratch,
+                                   int64_t n_trial, int64_t n_frame, void* stream);
+int seqik_head_affine_backward_f64(const double* head, const double* thorax, int64_t n_thorax_kp, const float* series,
+                                   const int32_t* counts, const float* consts, const float* affine, const float* grad_affine,
+                                   double* grad_head, double* grad_thorax, float* grad_consts, uint32_t* scratch,
+                                   int64_t n_trial, int64_t n_frame, void* stream);
 
 /* Shape-preserving cubic (pchip) resampling of uniformly sampled series onto a finer or coarser uniform grid: the hand-off
  * of joint angles to a simulation time step.  Replaces utils.interpolate_signal / interpolate_joint_angles

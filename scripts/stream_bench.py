@@ -2,7 +2,7 @@
 
 Algorithmic bytes per unit (DESIGN.md 5.3): fk 28+12+108 B/leg-frame (origin per frame), fk backward 28+108 in and 28+12
 (+16 with the lengths) out, head 48+28 B/frame (+12 with a
-per-frame neck), head backward 48+28 in and 48+12 out, pchip n+m values per block row and channel, pchip backward n+m in
+per-frame neck), head backward 48+28 in and 48+12 out, head_apply backward 24+24 in and 24+32 out, pchip n+m values per block row and channel, pchip backward n+m in
 and n out, align_apply 60+60 B/leg-frame, align_apply backward 60+60 in and 60+32 out, leg_affine backward 60 B read twice
 (fused path; the long path writes 28 B of keys and reads them in the select's four passes and the frame sweep), leg_series 60 in + 28 out, mid_quantile 4 B/element read (4 ranks x
 4 radix passes re-read the series: from L2 when it fits)."""
@@ -144,6 +144,73 @@ del g_head, r_req, l_req, r64, l64, n64, g64
 th = torch.randn((n_trial, 6 * n_frame, 3, 3), device="cuda", generator=g); hc = torch.rand((n_trial, 5), device="cuda", generator=g) + 0.5
 report("head_affine (series fp64 + radix select + affine)", timeit(lambda: engine.head_affine(r, th, hc)), nf * (24 + 36 + 20 + 20), nf, "frames")
 report("head_apply_kernel", timeit(lambda: engine.head_apply(r, torch.rand((n_trial, 8), device="cuda") + 0.5)), nf * 48, nf, "frames")
+# head alignment backward: apply backward (head + dL/dout in, dL/dhead + per-frame dL/daffine rows out, + the frame sum); the
+# statistics backward alone (the forward's series and counts kept, as autograd keeps them): 20 B of series read per frame
+# (twice on the long path, which writes and re-reads 20 B of keys), the scattered contributions per trial; forward + backward
+# through autograd; and the same VJP through torch autograd of the head alignment in float32 torch ops with torch.nanquantile
+aff_h, _, series_h = engine._head_affine(torch, r, th, hc, 5e-5)
+counts_h = engine.head_affine(r, th, hc)[1].flatten()
+g_ha = torch.randn(r.shape, device="cuda", generator=g)
+h_ha = torch.randn((n_trial, 8), device="cuda", generator=g)
+report("head_apply_backward (tile kernel + frame sum)", timeit(lambda: engine.head_apply_backward(r, aff_h, g_ha)), nf * (24 + 24 + 24 + 32), nf, "frames")
+gh_buf, gt_buf = torch.zeros_like(r), torch.zeros_like(th)
+vjp = lambda hd, t, k, a, s, c, gh, gt: engine._head_affine_vjp(torch, hd, t, k, a, h_ha[:hd.shape[0]].contiguous(), s, c, gh, gt, True, True)
+report(f"head_affine_backward statistics ({n_trial} x {6 * n_frame}: long path)",
+       timeit(lambda: vjp(r, th, hc, aff_h, series_h, counts_h, gh_buf, gt_buf)), nf * (20 + 20 + 20), nf, "frames")
+r_f, th_f = r.view(6 * n_trial, n_frame, 2, 3), th.view(6 * n_trial, n_frame, 3, 3)       # the same frames as 1000-frame trials
+hc_f = hc.repeat(6, 1)
+aff_f, _, series_f = engine._head_affine(torch, r_f, th_f, hc_f, 5e-5)
+counts_f = engine.head_affine(r_f, th_f, hc_f)[1].flatten()
+h_ha = torch.randn((6 * n_trial, 8), device="cuda", generator=g)
+report("head_affine (series fp64 + radix select + affine), 6000 x 1000", timeit(lambda: engine.head_affine(r_f, th_f, hc_f)), nf * (24 + 36 + 20 + 20), nf, "frames")
+report(f"head_affine_backward statistics ({6 * n_trial} x {n_frame}: fused path)",
+       timeit(lambda: vjp(r_f, th_f, hc_f, aff_f, series_f, counts_f, gh_buf.view(r_f.shape), gt_buf.view(th_f.shape))), nf * 20, nf, "frames")
+r_req, th_req = r_f.clone().requires_grad_(), th_f.clone().requires_grad_()
+report("head_apply(head_affine) + backward through autograd (kernels, 6000 x 1000)",
+       timeit(lambda: torch.autograd.grad(engine.head_apply(r_req, engine.head_affine(r_req, th_req, hc_f)[0]), [r_req, th_req],
+                                          g_ha.view(r_f.shape))),
+       nf * (24 + 36 + 20 + 20 + 24 + 24 + 24 + 24 + 32 + 20 + 24 + 36), nf, "frames")
+
+
+def torch_head_align(hd, t, k, thr=5e-5):
+    base, tip = hd[:, :, 0], hd[:, :, 1]
+    d = torch.linalg.vector_norm(base - 0.5 * (t[:, :, 0] + t[:, :, -1]), dim=-1)
+    with torch.no_grad():
+        dd = (d[:, 2:] - d[:, 1:-1]) - (d[:, 1:-1] - d[:, :-2])
+        still = torch.cat([dd < thr, torch.zeros_like(dd[:, :2], dtype=torch.bool)], dim=1)
+    nan = torch.full_like(d, float("nan"))
+    series = torch.stack([torch.where(still, base[..., c], nan) for c in range(3)]
+                         + [torch.where(still, d, nan), torch.linalg.vector_norm(tip - base, dim=-1)], dim=1)
+    q = torch.nanquantile(series, torch.tensor([0.45, 0.55], device=hd.device), dim=2).mean(0)           # (trial, 5)
+    o = q[:, None, :3]
+    b = (base - o) * (k[:, 3:4] / q[:, 3:4])[:, None] + k[:, None, :3]
+    tp = (tip - o) * (k[:, 4:5] / q[:, 4:5])[:, None] + k[:, None, :3]
+    return torch.stack([b, tp], dim=2)
+
+
+def torch_head_vjp():                                             # torch.nanquantile takes at most 2^24 values per call
+    for c0 in range(0, 6 * n_trial, 3000):
+        sl = slice(c0, c0 + 3000)
+        torch.autograd.grad(torch_head_align(r_req[sl], th_req[sl], hc_f[sl]), [r_req, th_req], g_ha.view(r_f.shape)[sl])
+
+
+report("float32 torch-ops head alignment (torch.nanquantile) + torch autograd VJP (reference point, 6000 x 1000)", timeit(torch_head_vjp, reps=3),
+       nf * (24 + 36 + 20 + 20 + 24 + 24 + 24 + 24 + 32 + 20 + 24 + 36), nf, "frames")
+del g_ha, gh_buf, gt_buf, r_req, th_req, series_h, series_f
+# the long path: 600 trials x 100 000 frames (series and keys through scratch), normal-random key points
+lh = torch.randn((600, 100000, 2, 3), device="cuda", generator=g)
+lt = torch.randn((600, 100000, 3, 3), device="cuda", generator=g)
+lk = hc[:600].contiguous()
+nf_long = 600 * 100000
+aff_l, _, series_l = engine._head_affine(torch, lh, lt, lk, 5e-5)
+counts_l = engine.head_affine(lh, lt, lk)[1].flatten()
+h_ha = torch.randn((600, 8), device="cuda", generator=g)
+gl_h, gl_t = torch.zeros_like(lh), torch.zeros_like(lt)
+report("head_affine long path (600 x 100 000)", timeit(lambda: engine.head_affine(lh, lt, lk), reps=5), nf_long * (24 + 36 + 20 + 20), nf_long, "frames")
+report("head_affine_backward long path (600 x 100 000): keys + select + frames + scatter",
+       timeit(lambda: vjp(lh, lt, lk, aff_l, series_l, counts_l, gl_h, gl_t), reps=5),
+       nf_long * (20 + 20 + 4 * 20 + 20), nf_long, "frames")
+del lh, lt, series_l, gl_h, gl_t
 # pchip resampler: the 6000 x 1000 x 7 angles of this workload from 100 Hz onto a 1 kHz grid (42e6 in, 420e6 out)
 for dt, nb in ((torch.float32, 4), (torch.float64, 8)):
     a = angles.to(dt)

@@ -12,7 +12,7 @@ import numpy as np
 _HERE = Path(__file__).resolve().parent
 LIB_PATH = _HERE / "csrc" / "libseqik_sm100.so"
 
-ABI_VERSION = 12
+ABI_VERSION = 13
 CHAIN_PARAM_FLOATS = 32
 FLAG_ESCAPE = 1 << 4
 FLAG_SKIP_CONFIRM = 1 << 5
@@ -60,6 +60,9 @@ _SIGNATURES = {
     "seqik_head_series_f64": (_int, [_vp, _vp, _i64, ctypes.c_double, _vp, _vp, _i64, _i64, _vp]),
     "seqik_head_affine_f32": (_int, [_vp, _vp, _vp, _i64, _vp]),
     "seqik_head_apply_f32": (_int, [_vp, _vp, _vp, _i64, _i64, _vp]),
+    "seqik_head_apply_backward_f32": (_int, [_vp, _vp, _vp, _vp, _vp, _i64, _i64, _vp]),
+    "seqik_head_affine_backward_f32": (_int, [_vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _vp]),
+    "seqik_head_affine_backward_f64": (_int, [_vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _vp]),
 }
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
 

@@ -286,8 +286,9 @@ def head_angles(r_head, l_head, neck, rest, affine_r=None, affine_l=None):
     carries a ``grad_fn`` whose backward is the ``seqik_head_angles_backward_f32`` kernel (see ``head_angles_backward``).
     An (n_trial, 3) neck gets the sum over frames; ``rest`` gets dL/drest[:, 0] = the sum of dL/dhead_pitch and
     dL/drest[:, 1] = minus the sums of dL/dantenna_pitch L and R.  The affine rows are constants of the backward: one
-    that requires grad raises ValueError.  First derivatives only: a second backward raises.  Without inputs that
-    require grad the call is the plain kernel launch."""
+    that requires grad raises ValueError.  To differentiate through the head alignment, align first and pass no rows:
+    ``head_angles(head_apply(raw, head_affine(raw, thorax, consts)[0]), ...)``.  First derivatives only: a second backward
+    raises.  Without inputs that require grad the call is the plain kernel launch."""
     torch = N.require_cuda()
     if torch.is_grad_enabled():
         if any(isinstance(t, torch.Tensor) and t.requires_grad for t in (affine_r, affine_l)):
@@ -578,9 +579,23 @@ def _align_functions():
 def head_affine(head, thorax, consts, threshold: float = 5e-5):
     """AlignPose.align_head statistics: head (n_trial, n_frame, 2, 3), thorax (n_trial, n_frame, k, 3) -- both float32
     or both float64 --, consts (n_trial, 5) float32 = template antenna base xyz, Antenna_mid_thorax, Antenna
-    -> affine (n_trial, 8) = (origin xyz, scale_base, template xyz, scale_tip), counts (n_trial, 5)."""
+    -> affine (n_trial, 8) = (origin xyz, scale_base, template xyz, scale_tip), counts (n_trial, 5).
+
+    Differentiable: when grad mode is on and ``head``, ``thorax`` or ``consts`` requires grad, ``affine`` carries a
+    ``grad_fn`` whose backward is the ``seqik_head_affine_backward`` kernel (see ``head_affine_backward``); the gradients
+    come back in the inputs' dtype and ``counts`` is not differentiable.  The stationary frames are held fixed as the
+    forward chose them, and each mid-quantile passes its gradient to the frames that hold its four order statistics
+    (ties: the first frames in frame order, include/seqik.h).  The differentiable route to the head angles is
+    ``head_angles(head_apply(raw, head_affine(raw, thorax, consts)[0]), ...)``.  First derivatives only: a second
+    backward raises.  Without inputs that require grad the call is the plain kernel launches."""
     torch = N.require_cuda()
-    lib = N.load_library()
+    if torch.is_grad_enabled() and any(isinstance(t, torch.Tensor) and t.requires_grad for t in (head, thorax, consts)):
+        return _head_align_functions()[0].apply(head, thorax, consts, float(threshold))
+    affine, counts, _ = _head_affine(torch, head, thorax, consts, threshold)
+    return affine, counts
+
+
+def _head_affine_inputs(torch, head, thorax, consts):
     dtype = head.dtype
     if dtype not in (torch.float32, torch.float64) or thorax.dtype != dtype:
         raise ValueError("head and thorax must both be float32 or both float64")
@@ -589,23 +604,101 @@ def head_affine(head, thorax, consts, threshold: float = 5e-5):
     if thorax.dim() != 4 or tuple(thorax.shape[:2]) != (n_trial, n_frame):
         raise ValueError("thorax must be (n_trial, n_frame, n_kp, 3)")
     thorax = _check(thorax, "thorax", (3,), dtype)
-    consts = _check(consts, "consts", (5,))
+    _check(consts, "consts", (5,))
+    return n_trial, n_frame
+
+
+def _head_series(torch, lib, head, thorax, threshold, n_trial, n_frame):
     dev = head.device
     series = torch.empty((n_trial * 5, n_frame), dtype=torch.float32, device=dev)
     counts = torch.empty((n_trial * 5,), dtype=torch.int32, device=dev)
-    affine = torch.empty((n_trial, 8), dtype=torch.float32, device=dev)
-    fn = lib.seqik_head_series_f32 if dtype == torch.float32 else lib.seqik_head_series_f64
+    fn = lib.seqik_head_series_f32 if head.dtype == torch.float32 else lib.seqik_head_series_f64
     with torch.cuda.device(dev):
-        st = N.stream_ptr(torch, dev)
         N.check(fn(N.ptr(head), N.ptr(thorax), int(thorax.shape[2]), float(threshold), N.ptr(series),
-                   N.ptr(counts), n_trial, n_frame, st), "seqik_head_series")
+                   N.ptr(counts), n_trial, n_frame, N.stream_ptr(torch, dev)), "seqik_head_series")
+    return series, counts
+
+
+def _head_affine(torch, head, thorax, consts, threshold):
+    """-> (affine (n_trial, 8), counts (n_trial, 5), series (n_trial * 5, n_frame)): the series and counts are what the
+    backward needs."""
+    lib = N.load_library()
+    n_trial, n_frame = _head_affine_inputs(torch, head, thorax, consts)
+    dev = head.device
+    series, counts = _head_series(torch, lib, head, thorax, threshold, n_trial, n_frame)
+    affine = torch.empty((n_trial, 8), dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev):
         stats = mid_quantile(series, counts)
-        N.check(lib.seqik_head_affine_f32(N.ptr(stats), N.ptr(consts), N.ptr(affine), n_trial, st), "seqik_head_affine_f32")
-    return affine, counts.view(n_trial, 5)
+        N.check(lib.seqik_head_affine_f32(N.ptr(stats), N.ptr(consts), N.ptr(affine), n_trial, N.stream_ptr(torch, dev)),
+                "seqik_head_affine_f32")
+    return affine, counts.view(n_trial, 5), series
+
+
+def _head_affine_vjp(torch, head, thorax, consts, affine, grad_affine, series, counts, grad_head, grad_thorax,
+                     want_thorax, want_consts):
+    lib = N.load_library()
+    n_trial, n_frame = _head_affine_inputs(torch, head, thorax, consts)
+    _check(affine, "affine", (8,))
+    grad_affine = _check(grad_affine, "grad_affine", (8,))
+    if tuple(affine.shape) != (n_trial, 8) or tuple(grad_affine.shape) != (n_trial, 8):
+        raise ValueError(f"affine and grad_affine must be ({n_trial}, 8)")
+    dev, dtype = head.device, head.dtype
+    if grad_head is None:
+        grad_head = torch.zeros_like(head)
+    elif grad_head.shape != head.shape:
+        raise ValueError(f"grad_head must be {tuple(head.shape)}")
+    else:
+        _check(grad_head, "grad_head", (2, 3), dtype)
+    if not want_thorax:
+        grad_thorax = None
+    elif grad_thorax is None:
+        grad_thorax = torch.zeros_like(thorax)
+    elif grad_thorax.shape != thorax.shape:
+        raise ValueError(f"grad_thorax must be {tuple(thorax.shape)}")
+    else:
+        _check(grad_thorax, "grad_thorax", (3,), dtype)
+    grad_consts = torch.empty((n_trial, 5), dtype=torch.float32, device=dev) if want_consts else None
+    scratch = None if n_frame <= 1024 else torch.empty((n_trial * 5 * (n_frame + 12),), dtype=torch.int32, device=dev)
+    fn = lib.seqik_head_affine_backward_f32 if dtype == torch.float32 else lib.seqik_head_affine_backward_f64
+    with torch.cuda.device(dev):
+        rc = fn(N.ptr(head), N.ptr(thorax), int(thorax.shape[2]), N.ptr(series), N.ptr(counts), N.ptr(consts), N.ptr(affine),
+                N.ptr(grad_affine), N.ptr(grad_head), N.ptr(grad_thorax), N.ptr(grad_consts), N.ptr(scratch), n_trial, n_frame,
+                N.stream_ptr(torch, dev))
+    N.check(rc, "seqik_head_affine_backward")
+    return grad_head, grad_thorax, grad_consts
+
+
+def head_affine_backward(head, thorax, consts, affine, grad_affine, threshold: float = 5e-5, grad_head=None, grad_thorax=None):
+    """Vector-Jacobian product of ``head_affine``: grad_affine (n_trial, 8) = dL/daffine -> (grad_head (n_trial, n_frame, 2, 3),
+    grad_thorax (n_trial, n_frame, k, 3), grad_consts (n_trial, 5)), the first two in the inputs' dtype.  ``affine`` is the
+    forward's result; the series and the stationary frames are recomputed with ``threshold``.  The statistics'
+    contributions are ADDED into ``grad_head`` / ``grad_thorax`` when they are given (e.g. the output of
+    ``head_apply_backward``; updated in place), else into zeros.  The frames, the tie rule and the float summation order
+    are those of include/seqik.h: the result is deterministic."""
+    torch = N.require_cuda()
+    lib = N.load_library()
+    n_trial, n_frame = _head_affine_inputs(torch, head, thorax, consts)
+    series, counts = _head_series(torch, lib, head, thorax, threshold, n_trial, n_frame)
+    return _head_affine_vjp(torch, head, thorax, consts, affine, grad_affine, series, counts, grad_head, grad_thorax, True, True)
 
 
 def head_apply(head, affine):
+    """The affine map of align_head (alignment.py:547-553) as a standalone pass: head (n_trial, n_frame, 2, 3) float32,
+    affine (n_trial, 8) = (origin xyz, scale_base, template xyz, scale_tip) -> aligned head (n_trial, n_frame, 2, 3) with
+    base' = (base - origin) * scale_base + template and tip' = (tip - origin) * scale_tip + template.
+
+    Differentiable: when grad mode is on and ``head`` or ``affine`` requires grad, the result carries a ``grad_fn`` whose
+    backward is the ``seqik_head_apply_backward_f32`` kernel (see ``head_apply_backward``).  Composed with ``head_affine``
+    under autograd, ``head_apply(head, head_affine(head, thorax, consts)[0])`` gives the full gradient with respect to the
+    raw antenna points, the thorax and the consts.  First derivatives only: a second backward raises.  Without inputs that
+    require grad the call is the plain kernel launch."""
     torch = N.require_cuda()
+    if torch.is_grad_enabled() and any(isinstance(t, torch.Tensor) and t.requires_grad for t in (head, affine)):
+        return _head_align_functions()[1].apply(head, affine)
+    return _head_apply(torch, head, affine)
+
+
+def _head_apply(torch, head, affine):
     lib = N.load_library()
     head = _check(head, "head", (2, 3))
     affine = _check(affine, "affine", (8,))
@@ -615,6 +708,75 @@ def head_apply(head, affine):
         rc = lib.seqik_head_apply_f32(N.ptr(head), N.ptr(affine), N.ptr(out), n_trial, n_frame, N.stream_ptr(torch, head.device))
     N.check(rc, "seqik_head_apply_f32")
     return out
+
+
+def head_apply_backward(head, affine, grad_out, want_head: bool = True, want_affine: bool = True):
+    """Vector-Jacobian product of ``head_apply``: grad_out (n_trial, n_frame, 2, 3) = dL/dout -> (grad_head (n_trial, n_frame,
+    2, 3) | None, grad_affine (n_trial, 8) | None).  grad_head is scale_base * grad_out for the bases and scale_tip * grad_out
+    for the tips; grad_affine is the sum over frames of the kernel's per-frame rows (include/seqik.h)."""
+    torch = N.require_cuda()
+    lib = N.load_library()
+    head = _check(head, "head", (2, 3))
+    affine = _check(affine, "affine", (8,))
+    if head.dim() != 4 or affine.dim() != 2 or affine.shape[0] != head.shape[0]:
+        raise ValueError("head must be (n_trial, n_frame, 2, 3) and affine (n_trial, 8)")
+    grad_out = _check(grad_out, "grad_out", (2, 3))
+    if grad_out.shape != head.shape:
+        raise ValueError(f"grad_out must be {tuple(head.shape)}, got {tuple(grad_out.shape)}")
+    n_trial, n_frame = int(head.shape[0]), int(head.shape[1])
+    dev = head.device
+    grad_head = torch.empty_like(head) if want_head else None
+    part = torch.empty((n_trial, n_frame, 8), dtype=torch.float32, device=dev) if want_affine else None
+    with torch.cuda.device(dev):
+        rc = lib.seqik_head_apply_backward_f32(N.ptr(head), N.ptr(affine), N.ptr(grad_out), N.ptr(grad_head), N.ptr(part),
+                                               n_trial, n_frame, N.stream_ptr(torch, dev))
+    N.check(rc, "seqik_head_apply_backward_f32")
+    return grad_head, (part.sum(dim=1) if want_affine else None)
+
+
+_HEAD_ALIGN_FUNCTIONS = None
+
+
+def _head_align_functions():
+    """The torch.autograd.Functions of head_affine and head_apply (built on first use: torch is imported lazily)."""
+    global _HEAD_ALIGN_FUNCTIONS
+    if _HEAD_ALIGN_FUNCTIONS is not None:
+        return _HEAD_ALIGN_FUNCTIONS
+    import torch
+    from torch.autograd.function import once_differentiable
+
+    class HeadAffine(torch.autograd.Function):
+        @staticmethod
+        def forward(ctx, head, thorax, consts, threshold):
+            affine, counts, series = _head_affine(torch, head, thorax, consts, threshold)
+            ctx.save_for_backward(head, thorax, consts, affine, series, counts)
+            ctx.mark_non_differentiable(counts)
+            return affine, counts
+
+        @staticmethod
+        @once_differentiable
+        def backward(ctx, grad_affine, _grad_counts):
+            head, thorax, consts, affine, series, counts = ctx.saved_tensors
+            need_head, need_thorax, need_consts = ctx.needs_input_grad[:3]
+            gh, gt, gk = _head_affine_vjp(torch, head, thorax, consts, affine, grad_affine.contiguous(), series, counts,
+                                          None, None, need_thorax, need_consts)
+            return (gh if need_head else None), gt, gk, None
+
+    class HeadApply(torch.autograd.Function):
+        @staticmethod
+        def forward(ctx, head, affine):
+            ctx.save_for_backward(head, affine)
+            return _head_apply(torch, head, affine)
+
+        @staticmethod
+        @once_differentiable
+        def backward(ctx, grad_out):
+            head, affine = ctx.saved_tensors
+            need_head, need_affine = ctx.needs_input_grad
+            return head_apply_backward(head, affine, grad_out.contiguous(), want_head=need_head, want_affine=need_affine)
+
+    _HEAD_ALIGN_FUNCTIONS = (HeadAffine, HeadApply)
+    return _HEAD_ALIGN_FUNCTIONS
 
 
 def pchip_resample(series, original_ts: float, new_ts: float):
